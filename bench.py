@@ -54,6 +54,9 @@ def parse():
                     help="'sharded': only the shape-sharded job (configs 3 / 5: --model, --shapes_per_gpu, --grid_res), shapes/s")
     ap.add_argument('--shapes_per_gpu', type=int, default=2)
     ap.add_argument('--skip_sharded', action='store_true', help='headline run without the sharded-job / tile-sharded sections')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write what the last timed step returned on rank 0 (voxel_index, sdf) as DIR/<name>.npy, for output-for-output "
+                         "comparison of two builds on the same seeded workload")
     return ap.parse_args()
 
 
@@ -178,6 +181,26 @@ def run_reference(args):
         line['cpu_baseline']['hosts'] = 1
         line['cpu_baseline']['sample'] += '; launched with %d ranks: rank 0 alone ran on this single host' % world
     print(json.dumps(line))
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy: floating arrays as float32, integer arrays as float64 (exact below 2^53).
+    The arrays share their first axis.  Above DUMP_LIMIT_BYTES in all, a fixed, seeded subset of rows is written instead,
+    with its row numbers as row_index.npy, so that runs with the same arguments dump the same rows."""
+    arrays = {k: np.asarray(a, np.float32 if np.issubdtype(a.dtype, np.floating) else np.float64) for k, a in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a.nbytes // max(n, 1) for a in arrays.values())
+    keep = DUMP_LIMIT_BYTES // (row_bytes + 8)
+    if n > keep:
+        rows = np.sort(np.random.RandomState(0).choice(n, keep, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays['row_index'] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
 
 
 def workload_config(args, Q):
@@ -387,17 +410,18 @@ def run_b200(args):
         if not host:
             eng.profile_enable(precision == 'tc')
         total_ms = 0.0
+        out = None
         for _ in range(steps):
             flush.zero_()
             torch.cuda.synchronize()
             if host:
                 t0 = time.perf_counter()
-                fn()
+                out = fn()
                 total_ms += (time.perf_counter() - t0) * 1e3     # the host call returns after its D2H completed
             else:
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 e0.record()
-                fn()
+                out = fn()
                 e1.record()
                 torch.cuda.synchronize()
                 total_ms += e0.elapsed_time(e1)
@@ -406,7 +430,7 @@ def run_b200(args):
         t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t.item()), launches
+        return float(t.item()), launches, out
 
     try:
         peaks_hbm = json.load(open(os.path.join(ROOT, 'MEASURED_PEAKS.json')))['hbm_gbs']
@@ -414,8 +438,10 @@ def run_b200(args):
         peaks_hbm = 6576.1   # B200_PROFILING.md fallback (measured copy bandwidth of this pool)
     sampler = ClockSampler(local_rank)
     sampler.start()
-    dev_ms, launches = timed(step_dev, args.steps, max(args.warmup, 3))
+    dev_ms, launches, (lin_last, sdf_last) = timed(step_dev, args.steps, max(args.warmup, 3))
     guard_total = eng.last_guard_count() if precision == 'tc' else 0   # warm-up + timed steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'voxel_index': lin_last.cpu().numpy(), 'sdf': sdf_last.cpu().numpy()})
 
     prof = eng.profile_get() if precision == 'tc' else None
     eng.profile_enable(False)
@@ -490,7 +516,7 @@ def run_b200(args):
             eng_fit.close()
         except Exception as e:  # noqa: BLE001
             tile_sharded = {'error': '%s: %s' % (type(e).__name__, e)}
-    e2e_ms, _ = timed(step_host, args.steps, 1, host=True)
+    e2e_ms, _, _ = timed(step_host, args.steps, 1, host=True)
     guard_frac = guard_total / max(Q * (args.steps + max(args.warmup, 3)), 1)
 
     q_total = torch.tensor([Q], dtype=torch.float64, device=dev)
