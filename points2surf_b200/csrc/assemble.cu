@@ -594,113 +594,12 @@ subsample_weighted_kernel(const float* __restrict__ pts, int N, const float* __r
     for (unsigned j = tid; n_direct + j < (unsigned)S; j += kThreads) out[q * S + n_direct + j] = s.cand_id[j];
 }
 
-// K3 by rejection: the same successive-sampling law with a quarter of the work when N >= 2 S.
-// Drawing without replacement with probabilities ~ w_i is: propose a point uniformly, accept it with probability w_i
-// (w_i <= 1), skip points that were already taken, repeat until S points are taken.  Proposal j of query q is a fixed
-// function of (seed, q, j) (Philox block j / 2 -> two (index, uniform) pairs), so the accepted set -- the first S distinct
-// accepted proposals in proposal order -- does not depend on how the proposals are spread over threads and rounds.
-// Only ~S / mean(w) * 1.1 ~ 3 400 of the points are touched per query instead of all 10 000 (plus one cheap pass for the
-// maximum distance), and there is no selection or sort.  s_first[i] = position of the first accepted proposal of point i.
-constexpr int kRejPer = 8;        // proposals per thread and round (first round); even
-constexpr int kRejRounds = 256;
-
-__global__ void __launch_bounds__(kThreads)
-subsample_reject_kernel(const float* __restrict__ pts, int N, const float* __restrict__ queries, int64_t qbase,
-                        const int32_t* __restrict__ qidx, int S, uint64_t seed, int32_t* __restrict__ out_ids,
-                        float* __restrict__ out_pts, int* __restrict__ err_flag) {
-    extern __shared__ int s_first[];             // [N]
-    __shared__ float redf[kThreads / 32];
-    __shared__ int redi[kThreads / 32];
-    __shared__ float s_dmax;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int64_t q = blockIdx.x;
-    const float qx = queries[q * 3 + 0], qy = queries[q * 3 + 1], qz = queries[q * 3 + 2];
-    const uint64_t qi = (uint64_t)(qbase + (qidx ? (int64_t)qidx[q] : q));
-    // max_i ||q - p_i|| in float32 like NumPy: sqrt is monotone, so it is the sqrt of the largest float32 squared sum
-    float m2 = 0.f;
-    for (int i = tid; i < N; i += kThreads) {
-        const float dx = __fsub_rn(qx, pts[i * 3 + 0]), dy = __fsub_rn(qy, pts[i * 3 + 1]), dz = __fsub_rn(qz, pts[i * 3 + 2]);
-        m2 = fmaxf(m2, __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz)));
-        s_first[i] = 0x7fffffff;
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) m2 = fmaxf(m2, __shfl_xor_sync(0xffffffffu, m2, o));
-    if (lane == 0) redf[warp] = m2;
-    __syncthreads();
-    if (tid == 0) {
-        float m = redf[0];
-        for (int w = 1; w < kThreads / 32; ++w) m = fmaxf(m, redf[w]);
-        s_dmax = __fsqrt_rn(m);
-    }
-    __syncthreads();
-    const float dmax = s_dmax;
-    int base = 0;                  // distinct accepted points so far
-    int pos0 = 0;                  // proposals consumed so far
-    int per = kRejPer;             // proposals per thread in this round (even, <= kRejPer)
-    for (int round = 0; round < kRejRounds; ++round) {
-        const int mypos = pos0 + tid * per;
-        int idx[kRejPer];
-        unsigned acc = 0;
-#pragma unroll
-        for (int e2 = 0; e2 < kRejPer / 2; ++e2) {
-            if (2 * e2 < per) {
-                uint32_t r[4];
-                philox4x32_10((uint32_t)seed, (uint32_t)(seed >> 32), (uint32_t)qi, (uint32_t)(qi >> 32), (uint32_t)((mypos >> 1) + e2), 0x9e3779b1u, r);
-#pragma unroll
-                for (int h = 0; h < 2; ++h) {
-                    const int i = (int)__umulhi(r[2 * h], (uint32_t)N);
-                    // dist_prob (utils.py:200-208) in float32 like NumPy
-                    const float d = norm_f32(__fsub_rn(qx, pts[i * 3 + 0]), __fsub_rn(qy, pts[i * 3 + 1]), __fsub_rn(qz, pts[i * 3 + 2]));
-                    const float w = fminf(fmaxf(__fsub_rn(1.0f, __fmul_rn(1.5f, __fdiv_rn(d, dmax))), 0.05f), 1.0f);
-                    const float u = (float)(r[2 * h + 1] >> 8) * (1.0f / 16777216.0f);     // [0, 1)
-                    idx[2 * e2 + h] = i;
-                    if (u < w) { acc |= 1u << (2 * e2 + h); atomicMin(&s_first[i], mypos + 2 * e2 + h); }
-                }
-            }
-        }
-        __syncthreads();
-        unsigned fresh = 0;
-#pragma unroll
-        for (int e = 0; e < kRejPer; ++e)
-            if (((acc >> e) & 1u) && s_first[idx[e]] == mypos + e) fresh |= 1u << e;
-        // exclusive prefix of the fresh counts in thread (= proposal) order
-        const int cnt = __popc(fresh);
-        int incl = cnt;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t; }
-        if (lane == 31) redi[warp] = incl;
-        __syncthreads();
-        int wbase = 0, total = 0;
-#pragma unroll
-        for (int w = 0; w < kThreads / 32; ++w) { const int c = redi[w]; if (w < warp) wbase += c; total += c; }
-        int slot = base + wbase + incl - cnt;
-#pragma unroll
-        for (int e = 0; e < kRejPer; ++e) {
-            if ((fresh >> e) & 1u) {
-                if (slot < S) {
-                    const int i = idx[e];
-                    out_ids[q * S + slot] = i;
-                    if (out_pts) {
-                        float* o = out_pts + (q * S + slot) * 3;
-                        o[0] = pts[i * 3 + 0]; o[1] = pts[i * 3 + 1]; o[2] = pts[i * 3 + 2];
-                    }
-                }
-                ++slot;
-            }
-        }
-        base += total;
-        if (base >= S) return;
-        pos0 += kThreads * per;
-        // size of the next round from this round's yield (deterministic: block-uniform integers only)
-        const long long need = ((long long)(S - base) * (kThreads * per) * 23 / 20) / (total > 0 ? total : 1) + 1;
-        const long long p2 = (need + 2 * kThreads - 1) / (2 * kThreads);
-        per = (int)(p2 < 1 ? 1 : (p2 > kRejPer / 2 ? kRejPer / 2 : p2)) * 2;
-        __syncthreads();       // redi is reused
-    }
-    if (tid == 0) atomicExch(err_flag, 2);
-}
-
-// K3 with a cell index: rejection sampling (see subsample_reject_kernel) whose proposals already follow the weights.
+// K3 with a cell index, by rejection: the same successive-sampling law with a fraction of the work when N >= 2 S.
+// Drawing without replacement with probabilities ~ w_i is: propose a point, accept it so that proposing-and-accepting point i
+// has probability ~ w_i, skip points that were already taken, repeat until S points are taken.  Proposal j of query q is a
+// fixed function of (seed, q, j) (Philox block j / 2 -> two (slot, uniform) pairs), so the accepted set -- the first S
+// distinct accepted proposals in proposal order -- does not depend on how the proposals are spread over threads and rounds,
+// and there is no selection or sort.
 // The cloud is binned once per shape into kCG^3 cells (points in cell order, a tight box per cell).  Per query, a cell's
 // weight bound wq_c >= max_{i in c} w_i follows from the distance to its box (w is non-increasing in the distance); a
 // proposal picks a cell with probability ~ count_c * wq_c and a point uniformly inside it -- ONE integer drawn uniformly
@@ -710,6 +609,8 @@ subsample_reject_kernel(const float* __restrict__ pts, int N, const float* __res
 // farthest corner beats the best first-point distance are scanned.  Bounds are quantised UP to multiples of 1/65535, so
 // every probability above is an exact integer ratio; 40 random bits select the slot (relative error of a point's
 // probability <= 2e-7).
+constexpr int kRejPer = 8;        // proposals per thread and round (upper bound); even
+constexpr int kRejRounds = 256;
 constexpr int kCG = 12, kCC = kCG * kCG * kCG;                 // 1728 cells
 constexpr int kCPT = (kCC + kThreads - 1) / kThreads;          // consecutive cells per thread (7)
 
@@ -881,7 +782,7 @@ subsample_cells_kernel(const CloudIndex ix, int N, const float* __restrict__ que
         if (c < kCC) { run += (uint32_t)cnt[k] * wq[k]; s_prefix[c] = run; s_wq[c] = (uint16_t)wq[k]; }
     }
     __syncthreads();
-    // ---- proposal rounds (same protocol as subsample_reject_kernel)
+    // ---- proposal rounds
     int base = 0, pos0 = 0, per = 6;
     for (int round = 0; round < kRejRounds; ++round) {
         const int mypos = pos0 + tid * per;
@@ -1043,10 +944,10 @@ void ball_patch(const float* pts, int64_t N, const float* queries, int64_t Q, in
 // Cell index of a cloud for the weighted sub-sampler: bounding box -> cell keys -> stable radix sort (points of a cell keep
 // their id order, so the result is deterministic) -> per-cell ranges, sorted points, tight boxes.  The index lives in a
 // thread-local workspace and is valid until the next call on this thread (stream order).
+constexpr size_t kSubsampleCacheBytes = 160 * 1024;   // dynamic shared memory of the cell and cached clock kernels: 4 B per point
+
 bool cloud_index_usable(int64_t N, int S, int mode) {
-    static int off = -1;
-    if (off < 0) { const char* e = getenv("P2S_SUBSAMPLE_NOCELLS"); off = (e && e[0] == '1') ? 1 : 0; }
-    return !off && mode == P2S_SUBSAMPLE_WEIGHTED && N >= 2 * (int64_t)S && (size_t)N * 4 <= 150 * 1024;
+    return mode == P2S_SUBSAMPLE_WEIGHTED && N >= 2 * (int64_t)S && (size_t)N * 4 <= kSubsampleCacheBytes;
 }
 
 const CloudIndex* cloud_index_build(const float* pts, int64_t N, cudaStream_t st) {
@@ -1093,32 +994,18 @@ void subsample(const float* pts, int64_t N, const float* queries, int64_t Q, int
         P2S_LAUNCH(subsample_uniform_kernel, (unsigned)cdiv(threads, 256), 256, 0, st, (int)N, Q, qbase, qidx, S, seed, out);
     } else if (mode == P2S_SUBSAMPLE_WEIGHTED) {
         const size_t cache_bytes = (size_t)N * sizeof(float);
-        static int no_reject = -1;
-        if (no_reject < 0) { const char* e = getenv("P2S_SUBSAMPLE_CLOCKS"); no_reject = (e && e[0] == '1') ? 1 : 0; }
-        if (cloud_index_usable(N, S, mode) && !no_reject) {
+        static thread_local bool attr_set = false;
+        if (!attr_set) {
+            P2S_CUDA(cudaFuncSetAttribute(subsample_cells_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSubsampleCacheBytes));
+            P2S_CUDA(cudaFuncSetAttribute(subsample_weighted_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSubsampleCacheBytes));
+            attr_set = true;
+        }
+        if (cloud_index_usable(N, S, mode)) {
+            // rejection over the cell index: cheap when at most half of the cloud is drawn
             if (!cidx) cidx = cloud_index_build(pts, N, st);
-            static thread_local bool attr_set = false;
-            if (!attr_set) {
-                P2S_CUDA(cudaFuncSetAttribute(subsample_cells_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 150 * 1024));
-                attr_set = true;
-            }
             P2S_LAUNCH(subsample_cells_kernel, (unsigned)Q, kThreads, cache_bytes, st, *cidx, (int)N, queries, qbase, qidx, S, seed, out, pts_out, err_flag_dev());
             gathered = true;
-        } else if (cache_bytes <= 160 * 1024 && N >= 2 * (int64_t)S && !no_reject) {
-            // rejection sampling: cheap when at most half of the cloud is drawn (the acceptance rate is >= 0.05 by construction)
-            static thread_local bool attr_set = false;
-            if (!attr_set) {
-                P2S_CUDA(cudaFuncSetAttribute(subsample_reject_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-                attr_set = true;
-            }
-            P2S_LAUNCH(subsample_reject_kernel, (unsigned)Q, kThreads, cache_bytes, st, pts, (int)N, queries, qbase, qidx, S, seed, out, pts_out, err_flag_dev());
-            gathered = true;
-        } else if (cache_bytes <= 160 * 1024) {
-            static thread_local bool attr_set = false;
-            if (!attr_set) {
-                P2S_CUDA(cudaFuncSetAttribute(subsample_weighted_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-                attr_set = true;
-            }
+        } else if (cache_bytes <= kSubsampleCacheBytes) {
             P2S_LAUNCH(subsample_weighted_kernel<true>, (unsigned)Q, kThreads, cache_bytes, st, pts, (int)N, queries, qbase, qidx, S, seed, out, err_flag_dev());
         } else {
             P2S_LAUNCH(subsample_weighted_kernel<false>, (unsigned)Q, kThreads, 0, st, pts, (int)N, queries, qbase, qidx, S, seed, out, err_flag_dev());

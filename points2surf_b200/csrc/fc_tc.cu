@@ -1,7 +1,7 @@
 // Tensor-core GEMM for the per-query FC tails of the TC path (QSTN/STN heads 1024->512->256->{4,4096} and the
-// decoder 1024->512 (x2), 1024->256, 256->128; source/points_to_surf_model.py:62-64,120-122,335,343,348-350):
-//     C[M][N] = act( A[M][K] * W[N][K]^T + b ),  A fp32 row-major, W pre-packed operand images, fp32 accumulation
-//     in TMEM, C fp32 row-major.
+// decoder 1024->512 (x2), 1024->256, 256->128; source/points_to_surf_model.py:62-64,120-122,335,343,348-350) and for
+// the training GEMMs:
+//     C[M][N] = act( A[M][K] * W[N][K]^T + b ),  W pre-packed operand images, fp32 accumulation in TMEM.
 // These layers produce the point rotation, the 64x64 feature transform and the logits, so they keep fp32-level
 // accuracy: every fp32 operand x is split into two fp16 numbers x_hi + x_lo (x_hi = fp16(x), x_lo = fp16(x - x_hi))
 // and the product is evaluated as A_hi*W_hi + A_lo*W_hi + A_hi*W_lo (the dropped lo*lo term is ~2^-22 relative).
@@ -32,15 +32,16 @@ struct FcBars {
     uint32_t tmem_base;
 };
 
-// A operand: fp32 rows (converted by the producer warps, `A`) or a pre-packed operand image `Aimg`
-// ([M/128][K/32][hi | lo][128 x 32 fp16], the W layout): then the producers have nothing to do and both operands of a k-step
-// arrive by bulk copy.  ncu showed the fp32 mode L1TEX-bound (61-77 % l1tex throughput, 17-19 % tensor-active): every A
-// element was loaded and split once per N tile (4x for the 1024->512 layers, 32x for the folded 256->4096 layer) through
-// row-per-thread loads.  pack_img == 3 writes C as the NEXT layer's operand image (k-steps out_kt_off.. of out_kt_total).
+// A operand: fp32 rows (converted by the producer warps, `A`; training GEMMs) or a pre-packed operand image `Aimg`
+// ([M/128][K/32][hi | lo][128 x 32 fp16], the W layout; FC tails): then the producers have nothing to do and both operands of
+// a k-step arrive by bulk copy.  ncu showed the fp32 mode L1TEX-bound on the FC tails (61-77 % l1tex throughput, 17-19 %
+// tensor-active): every A element was loaded and split once per N tile (4x for the 1024->512 layers, 32x for the folded
+// 256->4096 layer) through row-per-thread loads.
+// out_mode: 0 fp32 rows (ldc), 1 / 2 the pass kernel's per-query operand image (fp16 / hi | lo), 3 the NEXT layer's operand
+// image (k-steps out_kt_off.. of out_kt_total).
 __global__ void __launch_bounds__(160) fc_tc_kernel(const float* __restrict__ A, int lda, const uint8_t* __restrict__ Wimg,
                                                     const float* __restrict__ bias, float* __restrict__ C, int ldc,
-                                                    int M, int N, int K, int relu, int pack_img,
-                                                    const float* __restrict__ in_bias, int in_relu,
+                                                    int M, int N, int K, int relu, int out_mode,
                                                     const uint8_t* __restrict__ Aimg, int out_kt_total, int out_kt_off) {
     extern __shared__ __align__(1024) uint8_t smem[];
     FcBars* bars = reinterpret_cast<FcBars*>(smem + kStages * (kStageA + kStageB));
@@ -81,15 +82,7 @@ __global__ void __launch_bounds__(160) fc_tc_kernel(const float* __restrict__ A,
             uint8_t* dst = smem + s * kStageA + (uint32_t)(tid >> 3) * 512u + (uint32_t)(tid & 7) * 16u;
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
-                float x[8] = {v[2 * c].x, v[2 * c].y, v[2 * c].z, v[2 * c].w, v[2 * c + 1].x, v[2 * c + 1].y, v[2 * c + 1].z, v[2 * c + 1].w};
-                if (in_bias) {          // A = act(A_raw + in_bias[k]): same fp32 operations as a separate bias / ReLU kernel
-                    const float4 b0 = __ldg(reinterpret_cast<const float4*>(in_bias + kt * kBK + c * 8)), b1 = __ldg(reinterpret_cast<const float4*>(in_bias + kt * kBK + c * 8 + 4));
-                    x[0] += b0.x; x[1] += b0.y; x[2] += b0.z; x[3] += b0.w; x[4] += b1.x; x[5] += b1.y; x[6] += b1.z; x[7] += b1.w;
-                    if (in_relu) {
-#pragma unroll
-                        for (int e = 0; e < 8; ++e) x[e] = fmaxf(x[e], 0.f);
-                    }
-                }
+                const float x[8] = {v[2 * c].x, v[2 * c].y, v[2 * c].z, v[2 * c].w, v[2 * c + 1].x, v[2 * c + 1].y, v[2 * c + 1].z, v[2 * c + 1].w};
                 uint32_t hi[4], lo[4];
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {
@@ -118,7 +111,7 @@ __global__ void __launch_bounds__(160) fc_tc_kernel(const float* __restrict__ A,
             uint32_t r[32];
             tmem_ld_x32(tmem + lane_base + n0, r);
             tmem_ld_wait();
-            if (pack_img == 3) {
+            if (out_mode == 3) {
                 // C as the next layer's A operand image: this 32-column chunk is exactly one k-step of that layer
                 uint8_t* blk = reinterpret_cast<uint8_t*>(C) + ((size_t)blockIdx.y * out_kt_total + out_kt_off + nt * 4 + (n0 >> 5)) * (size_t)kStageA +
                                (uint32_t)(tid >> 3) * 512u + (uint32_t)(tid & 7) * 16u;
@@ -139,11 +132,11 @@ __global__ void __launch_bounds__(160) fc_tc_kernel(const float* __restrict__ A,
                     *reinterpret_cast<uint4*>(blk + g * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
                     *reinterpret_cast<uint4*>(blk + kHalf + g * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
                 }
-            } else if (row < M && pack_img) {
+            } else if (row < M && out_mode) {
                 // C is a per-row fp16 operand image of a [64][64] matrix (row-major index = column of this GEMM):
                 // K-major, LBO 128, SBO 1024 -- the per-query B operand of the pass kernel
-                // pack_img == 2: split precision, 16384 B per row: hi image | lo image
-                uint8_t* img = reinterpret_cast<uint8_t*>(C) + (size_t)row * (pack_img == 2 ? 16384 : 8192);
+                // out_mode == 2: split precision, 16384 B per row: hi image | lo image
+                uint8_t* img = reinterpret_cast<uint8_t*>(C) + (size_t)row * (out_mode == 2 ? 16384 : 8192);
 #pragma unroll
                 for (int j = 0; j < 32; j += 8) {
                     const int col = nt * 128 + n0 + j;
@@ -158,7 +151,7 @@ __global__ void __launch_bounds__(160) fc_tc_kernel(const float* __restrict__ A,
                     }
                     const uint32_t off = (uint32_t)(o >> 3) * 1024u + (uint32_t)(i >> 3) * 128u + (uint32_t)(o & 7) * 16u;
                     *reinterpret_cast<uint4*>(img + off) = make_uint4(v[0], v[1], v[2], v[3]);
-                    if (pack_img == 2) *reinterpret_cast<uint4*>(img + 8192 + off) = make_uint4(vl[0], vl[1], vl[2], vl[3]);
+                    if (out_mode == 2) *reinterpret_cast<uint4*>(img + 8192 + off) = make_uint4(vl[0], vl[1], vl[2], vl[3]);
                 }
             } else if (row < M) {
 #pragma unroll
@@ -230,19 +223,6 @@ __global__ void __launch_bounds__(160) fc_tc_kernel(const float* __restrict__ A,
     if (warp == 4) tmem_dealloc(tmem, 128);
 }
 
-// fp32 W[N][K] -> images [N/128][K/32][hi | lo][128 x 32 fp16, K-major, LBO 128, SBO 512]
-__global__ void pack_fc_kernel(const float* __restrict__ W, int N, int K, uint8_t* __restrict__ img) {
-    int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= (int64_t)N * K) return;
-    int n = (int)(e / K), k = (int)(e % K);
-    int nt = n >> 7, r = n & 127, kt = k / kBK, kk = k % kBK;
-    size_t off = ((size_t)nt * (K / kBK) + kt) * kStageB + (size_t)(r >> 3) * 512 + (size_t)(kk >> 3) * 128 + (size_t)(r & 7) * 16 + (size_t)(kk & 7) * 2;
-    const float w = W[e];
-    const __half h = __float2half_rn(w);
-    *reinterpret_cast<__half*>(img + off) = h;
-    *reinterpret_cast<__half*>(img + off + kHalf) = __float2half_rn(w - __half2float(h));
-}
-
 // fp32 activations A[M][K] (+ optional bias / ReLU) -> A operand images [ceil(M/128)][K/32][hi | lo][128 x 32 fp16, K-major,
 // LBO 128, SBO 512]; rows >= M are zero.  One CTA per (row tile, k-step): 8 lanes read one row's 128 bytes (coalesced).
 __global__ void __launch_bounds__(256) pack_a_kernel(const float* __restrict__ A, int lda, int M, int K, const float* __restrict__ in_bias,
@@ -269,7 +249,7 @@ __global__ void __launch_bounds__(256) pack_a_kernel(const float* __restrict__ A
     }
 }
 
-// same image for N rows padded with zeros to Npad (multiple of 128)
+// fp32 W[N][K] -> images [Npad/128][K/32][hi | lo][128 x 32 fp16, K-major, LBO 128, SBO 512], rows N..Npad-1 zero
 __global__ void pack_fc_pad_kernel(const float* __restrict__ W, int N, int Npad, int K, uint8_t* __restrict__ img) {
     int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= (int64_t)Npad * K) return;
@@ -286,14 +266,7 @@ __global__ void pack_fc_pad_kernel(const float* __restrict__ W, int N, int Npad,
 
 bool fc_tc_supported(int N, int K) { return (N % 128 == 0) && (K % kBK == 0) && N >= 128 && K >= kBK; }
 
-uint8_t* fc_tc_pack(const Layer& L, std::vector<void*>& allocs) {
-    P2S_CHECK(fc_tc_supported(L.cout, L.cin), "layer shape not supported by the tensor-core FC kernel");
-    void* p = nullptr;
-    P2S_CUDA(cudaMalloc(&p, (size_t)L.cout * L.cin * 4));
-    allocs.push_back(p);
-    P2S_LAUNCH(pack_fc_kernel, (unsigned)cdiv((int64_t)L.cout * L.cin, 256), 256, 0, 0, L.W, L.cout, L.cin, (uint8_t*)p);
-    return (uint8_t*)p;
-}
+uint8_t* fc_tc_pack(const Layer& L, std::vector<void*>& allocs) { return fc_tc_pack_raw(L.W, L.cout, L.cin, allocs); }
 
 void fc_tc_init() {
     static bool done = false;
@@ -303,18 +276,15 @@ void fc_tc_init() {
     }
 }
 
+// A as fp32 rows, C as fp32 rows; N may end in a partial 128-column tile (N % 4 == 0)
 void launch_fc_tc(const float* A, int lda, const uint8_t* Wimg, const float* bias, float* C, int ldc,
-                  int64_t M, int N, int K, bool relu, cudaStream_t st, int pack_img, const float* in_bias, bool in_relu) {
+                  int64_t M, int N, int K, bool relu, cudaStream_t st) {
     if (M <= 0) return;
-    const bool padded_ok = !pack_img && N % 4 == 0 && N >= 64 && K % kBK == 0;   // partial last N tile (training GEMMs)
-    P2S_CHECK((fc_tc_supported(N, K) || padded_ok) && lda % 4 == 0 && (pack_img ? N == 4096 : ldc % 4 == 0), "bad FC shape for the tensor-core kernel");
+    P2S_CHECK(N % 4 == 0 && N >= 64 && K % kBK == 0 && K >= kBK && lda % 4 == 0 && ldc % 4 == 0, "bad FC shape for the tensor-core kernel");
     P2S_CHECK(cdiv(M, 128) <= 65535, "too many rows for one launch");
     dim3 grid((unsigned)cdiv(N, 128), (unsigned)cdiv(M, 128), 1);
-    P2S_LAUNCH(fc_tc_kernel, grid, 160, kFcSmem, st, A, lda, Wimg, bias, C, ldc, (int)M, N, K, relu ? 1 : 0, pack_img, in_bias, in_relu ? 1 : 0,
-               (const uint8_t*)nullptr, 0, 0);
+    P2S_LAUNCH(fc_tc_kernel, grid, 160, kFcSmem, st, A, lda, Wimg, bias, C, ldc, (int)M, N, K, relu ? 1 : 0, 0, (const uint8_t*)nullptr, 0, 0);
 }
-
-size_t fc_tc_a_image_bytes(int64_t M, int K) { return (size_t)cdiv(M, 128) * (size_t)(K / kBK) * kStageA; }
 
 void launch_pack_a(const float* A, int lda, int64_t M, int K, const float* in_bias, bool in_relu, uint8_t* img, cudaStream_t st) {
     if (M <= 0) return;
@@ -333,7 +303,7 @@ void launch_fc_tc_img(const uint8_t* Aimg, const uint8_t* Wimg, const float* bia
     P2S_CHECK(cdiv(M, 128) <= 65535, "too many rows for one launch");
     dim3 grid((unsigned)(N / 128), (unsigned)cdiv(M, 128), 1);
     P2S_LAUNCH(fc_tc_kernel, grid, 160, kFcSmem, st, (const float*)nullptr, 0, Wimg, bias, reinterpret_cast<float*>(C), ldc, (int)M, N, K, relu ? 1 : 0,
-               out_mode, (const float*)nullptr, 0, Aimg, out_kt_total, out_kt_off);
+               out_mode, Aimg, out_kt_total, out_kt_off);
 }
 
 // images of a raw fp32 matrix W[N][K] (device pointer)
@@ -342,19 +312,14 @@ uint8_t* fc_tc_pack_raw(const float* W, int N, int K, std::vector<void*>& allocs
     void* p = nullptr;
     P2S_CUDA(cudaMalloc(&p, (size_t)N * K * 4));
     allocs.push_back(p);
-    P2S_LAUNCH(pack_fc_kernel, (unsigned)cdiv((int64_t)N * K, 256), 256, 0, 0, W, N, K, (uint8_t*)p);
+    P2S_LAUNCH(pack_fc_pad_kernel, (unsigned)cdiv((int64_t)N * K, 256), 256, 0, 0, W, N, N, K, (uint8_t*)p);
     return (uint8_t*)p;
 }
 
 // Split-precision tensor-core GEMM for weights that change between calls (training): packs W [N][K] into a reusable
 // scratch image on `st`, then runs fc_tc_kernel.  Stream order makes the scratch reuse safe.  bias may be null.
 bool gemm_nt_tc_ok(const float* A, int lda, const float* C, int ldc, int64_t M, int N, int K) {
-    static int disabled = -1;
-    if (disabled < 0) {
-        const char* e = getenv("P2S_TRAIN_GEMM_FP32");
-        disabled = (e && e[0] == '1') ? 1 : 0;
-    }
-    return !disabled && N % 4 == 0 && N >= 64 && K % kBK == 0 && K >= kBK && N <= 4096 && M >= 128 && M < (int64_t)1 << 31 && lda % 4 == 0 && ldc % 4 == 0 &&
+    return N % 4 == 0 && N >= 64 && K % kBK == 0 && K >= kBK && N <= 4096 && M >= 128 && M < (int64_t)1 << 31 && lda % 4 == 0 && ldc % 4 == 0 &&
            ((uintptr_t)A % 16 == 0) && ((uintptr_t)C % 16 == 0);
 }
 
@@ -374,7 +339,7 @@ void launch_gemm_nt_tc(const float* A, int lda, const float* W, const float* bia
         bias = z;
     }
     P2S_LAUNCH(pack_fc_pad_kernel, (unsigned)cdiv((int64_t)Npad * K, 256), 256, 0, st, W, N, Npad, K, wimg);
-    launch_fc_tc(A, lda, wimg, bias, C, ldc, M, N, K, relu, st, 0);
+    launch_fc_tc(A, lda, wimg, bias, C, ldc, M, N, K, relu, st);
 }
 
 }  // namespace p2s

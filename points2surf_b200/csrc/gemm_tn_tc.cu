@@ -151,12 +151,7 @@ gemm_tn_tc_kernel(const float* __restrict__ A, int lda, const float* __restrict_
 }  // namespace
 
 bool gemm_tn_tc_ok(const float* A, int lda, const float* B, int ldb, int64_t M, int N, int K) {
-    static int disabled = -1;
-    if (disabled < 0) {
-        const char* e = getenv("P2S_TRAIN_GEMM_FP32");
-        disabled = (e && e[0] == '1') ? 1 : 0;
-    }
-    return !disabled && M >= 4096 && N >= 64 && K >= 64 && N % 4 == 0 && K % 4 == 0 && lda % 4 == 0 && ldb % 4 == 0 &&
+    return M >= 4096 && N >= 64 && K >= 64 && N % 4 == 0 && K % 4 == 0 && lda % 4 == 0 && ldb % 4 == 0 &&
            ((uintptr_t)A % 16 == 0) && ((uintptr_t)B % 16 == 0);
 }
 

@@ -71,10 +71,8 @@ bool fc_tc_supported(int N, int K);
 uint8_t* fc_tc_pack(const Layer& L, std::vector<void*>& allocs);
 void fc_tc_init();
 void launch_fc_tc(const float* A, int lda, const uint8_t* Wimg, const float* bias, float* C, int ldc,
-                  int64_t M, int N, int K, bool relu, cudaStream_t st, int pack_img = 0, const float* in_bias = nullptr,
-                  bool in_relu = false);
+                  int64_t M, int N, int K, bool relu, cudaStream_t st);
 uint8_t* fc_tc_pack_raw(const float* W, int N, int K, std::vector<void*>& allocs);
-size_t fc_tc_a_image_bytes(int64_t M, int K);
 void launch_pack_a(const float* A, int lda, int64_t M, int K, const float* in_bias, bool in_relu, uint8_t* img, cudaStream_t st);
 void launch_fc_tc_img(const uint8_t* Aimg, const uint8_t* Wimg, const float* bias, void* C, int ldc, int64_t M, int N, int K,
                       bool relu, cudaStream_t st, int out_mode, int out_kt_total = 0, int out_kt_off = 0);

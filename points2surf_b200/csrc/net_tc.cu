@@ -21,7 +21,8 @@
 // epilogue of the big layer; warp 8 issues the big-layer MMAs (blocking waits), warp 13 the mid-layer MMAs of both
 // chains (polling).
 //
-// The small per-query FC tails between the passes run as fp32 FMA GEMMs (net_fp32.cu kernels).
+// The small per-query FC tails between the passes run on the split-precision tensor-core FC kernel (fc_tc.cu) as a chain of
+// operand images; only the 256 -> 4 QSTN output layer and the 128 -> 2 logits layer stay on the fp32 FMA GEMM (net_fp32.cu).
 #include "model.cuh"
 #include "tc_ptx.cuh"
 
@@ -86,7 +87,7 @@ struct PassParams {
     int perq_layer;            // index of the mid layer with per-query weights, or -1
     const uint8_t* perq_img;   // [B] x 8192 B (precise: hi | lo, 16384 B)
     const uint8_t* w3_img;     // [8 chunks][32768 B] (precise: [8][hi | lo])  (K-major, LBO 128, SBO 2048)
-    float* out;                // [B,1024] raw max (bias / ReLU applied by the consumer: the FC kernel's producers add it on load)
+    float* out;                // [B,1024] raw max (bias / ReLU applied by the consumer: launch_pack_a adds it while packing)
     long long* wstats;         // diagnostics: per-role barrier wait cycles (null = off)
 };
 
@@ -554,55 +555,6 @@ __global__ void pack_kmajor_kernel(const float* __restrict__ W, int rows, int K,
     *reinterpret_cast<__half*>(img + off) = lo ? __float2half_rn(w - __half2float(h)) : h;
 }
 
-// per-query W1*T (fp32 [B][64][64], row = output channel) -> fp16 images of 8192 B
-__global__ void pack_perq_kernel(const float* __restrict__ W, int64_t B, uint8_t* __restrict__ img) {
-    int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= B * 4096) return;
-    int64_t b = e >> 12;
-    int r = (int)((e >> 6) & 63), k = (int)(e & 63);
-    uint32_t off = (uint32_t)(r >> 3) * 1024u + (uint32_t)(k >> 3) * 128u + (uint32_t)(r & 7) * 16u + (uint32_t)(k & 7) * 2u;
-    *reinterpret_cast<__half*>(img + b * 8192 + off) = __float2half_rn(W[e]);
-}
-
-// Fused per-query fold: img[b] = fp16 operand image of W1 * (T[b] + I), T[b] = the STN's raw fc3 output
-// viewed as [64][64] (model.py:66-68,196,201).  One CTA per query, 256 threads, W1 and T staged in shared memory.
-__global__ void __launch_bounds__(256) fold_w1_kernel(const float* __restrict__ W1, const float* __restrict__ T, int64_t B, uint8_t* __restrict__ img) {
-    __shared__ float sW[64][65];
-    __shared__ __align__(16) float sT[64][68];
-    const int64_t b = blockIdx.x;
-    const int tid = threadIdx.x;
-    for (int e = tid; e < 4096; e += 256) {
-        const int r = e >> 6, c = e & 63;
-        sW[r][c] = W1[e];
-        sT[r][c] = T[b * 4096 + e] + (r == c ? 1.0f : 0.0f);
-    }
-    __syncthreads();
-    // thread -> output row o = tid / 4, 16 consecutive input columns i0 = (tid % 4) * 16
-    const int o = tid >> 2, i0 = (tid & 3) * 16;
-    float acc[16];
-#pragma unroll
-    for (int i = 0; i < 16; ++i) acc[i] = 0.f;
-    for (int j = 0; j < 64; ++j) {
-        const float w = sW[o][j];
-#pragma unroll
-        for (int i4 = 0; i4 < 4; ++i4) {
-            const float4 t4 = *reinterpret_cast<const float4*>(&sT[j][i0 + 4 * i4]);
-            acc[4 * i4 + 0] = fmaf(w, t4.x, acc[4 * i4 + 0]);
-            acc[4 * i4 + 1] = fmaf(w, t4.y, acc[4 * i4 + 1]);
-            acc[4 * i4 + 2] = fmaf(w, t4.z, acc[4 * i4 + 2]);
-            acc[4 * i4 + 3] = fmaf(w, t4.w, acc[4 * i4 + 3]);
-        }
-    }
-    uint8_t* dst = img + b * 8192 + (uint32_t)(o >> 3) * 1024u + (uint32_t)(o & 7) * 16u;
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-        uint32_t v[4];
-#pragma unroll
-        for (int e = 0; e < 4; ++e) v[e] = pack_half2(acc[h * 8 + 2 * e], acc[h * 8 + 2 * e + 1]);
-        *reinterpret_cast<uint4*>(dst + (uint32_t)(i0 / 8 + h) * 128u) = make_uint4(v[0], v[1], v[2], v[3]);
-    }
-}
-
 // conv1 folded into the STN's last layer: W1*(T+I) with T = view(fc3(f) + b, 64, 64) is linear in f, so
 //   (W1*(T+I))[o][i] = sum_k f[k] * G[o*64+i][k] + g0[o*64+i],
 //   G[o*64+i][k] = sum_j W1[o][j] * Wfc3[j*64+i][k],   g0[o*64+i] = sum_j W1[o][j] * bfc3[j*64+i] + W1[o][i].
@@ -620,15 +572,6 @@ __global__ void fold_fc3_kernel(const float* __restrict__ W1, const float* __res
         for (int j = 0; j < 64; ++j) b = fmaf(W1[o * 64 + j], bfc3[j * 64 + i], b);
         g0[oi] = b;
     }
-}
-
-// out[b][i][j] = in[b][j][i] for 64x64 blocks (the STN's transform, transposed for the W1*T product)
-__global__ void transpose64_kernel(const float* __restrict__ in, float* __restrict__ out, int64_t B) {
-    int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= B * 4096) return;
-    int64_t b = e >> 12;
-    int i = (int)((e >> 6) & 63), j = (int)(e & 63);
-    out[e] = in[b * 4096 + j * 64 + i];
 }
 
 __global__ void guard_flag_kernel(const float* __restrict__ logits, int64_t B, float band, int32_t* __restrict__ list, int* __restrict__ count, int64_t base, int64_t cap) {
@@ -668,21 +611,22 @@ struct TcStack {           // one conv stack ending in the 128 -> 1024 layer
     const float* b3 = nullptr;
 };
 
-struct TcFc {                 // one Linear layer: fp32 weights + (optional) tensor-core operand images
-    const Layer* L = nullptr;
-    const uint8_t* img = nullptr;
+struct TcStnFc {              // tensor-core operand images of an STN's fc1 (1024 -> 512) and fc2 (512 -> 256)
+    const uint8_t* fc1 = nullptr;
+    const uint8_t* fc2 = nullptr;
 };
-struct TcStnFc { TcFc fc1, fc2, fc3; };
 
 struct TcWeights {
     TcStack qstn;                // pass A
     TcStack stn[2], fin[2];      // [0] local, [1] global: pass B, pass C
     TcStnFc qstn_fc, stn_fc[2];
-    TcFc head_fc1[2], head_fc2, head_fc3;
+    // decoder images: fc1_local / fc1_global (1024 -> 512), fc2 (1024 -> 256), fc3 (256 -> 128)
+    const uint8_t* head_fc1[2] = {nullptr, nullptr};
+    const uint8_t* head_fc2 = nullptr;
+    const uint8_t* head_fc3 = nullptr;
     // conv1 folded into stn2.fc3 per branch: images of G [4096 x 256] and bias g0 [4096]
     const uint8_t* fold_img[2] = {nullptr, nullptr};
     const float* fold_bias[2] = {nullptr, nullptr};
-    bool fc_on_tc = true;
     std::vector<void*> allocs;
     int sm_count = 148;
     // profile of the dominant kernel (bench.py roofline)
@@ -793,30 +737,6 @@ void launch_pass(Model& m, const TcStack& s, const Seg& s0, const Seg& s1, const
 
 Seg make_seg(const float* ptr, int n, int center) { return Seg{ptr, n, n > 0 ? (n + kTile - 1) / kTile : 0, center}; }
 
-// in_bias (optional, tensor-core kernel only): the layer reads act(in + in_bias) -- the raw max features of a pass get their
-// conv3 bias (and the STN's ReLU) on the way into the first FC layer instead of in separate copy / bias kernels
-void run_fc(const TcFc& f, const float* in, int lda, float* out, int ldc, int64_t Bc, bool relu, bool on_tc, cudaStream_t st,
-            const float* in_bias = nullptr, bool in_relu = false) {
-    const Layer& L = *f.L;
-    if (on_tc && f.img) launch_fc_tc(in, lda, f.img, L.b, out, ldc, Bc, L.cout, L.cin, relu, st, 0, in_bias, in_relu);
-    else {
-        P2S_CHECK(!in_bias, "input bias needs the tensor-core FC kernel");
-        launch_gemm_nt(in, 0, lda, L.W, 0, L.b, out, 0, ldc, (int)Bc, L.cout, L.cin, 1, relu, st);
-    }
-}
-
-void fc_tail(const Layer& b3src, const TcStnFc& s, bool on_tc, const float* gmax_raw, int64_t Bc, float* g, float* f1, float* f2, float* out, cudaStream_t st) {
-    // g = relu(max + b3) ; fc1 ; fc2 ; fc3     (model.py:44-64 / 103-122)
-    if (on_tc && s.fc1.img) run_fc(s.fc1, gmax_raw, 1024, f1, 512, Bc, true, true, st, b3src.b, true);
-    else {
-        P2S_CUDA(cudaMemcpyAsync(g, gmax_raw, (size_t)Bc * 1024 * 4, cudaMemcpyDeviceToDevice, st));
-        launch_bias_act(g, b3src.b, Bc, 1024, true, st);
-        run_fc(s.fc1, g, 1024, f1, 512, Bc, true, on_tc, st);
-    }
-    run_fc(s.fc2, f1, 512, f2, 256, Bc, true, on_tc, st);
-    run_fc(s.fc3, f2, 256, out, s.fc3.L->cout, Bc, false, on_tc, st);
-}
-
 }  // namespace
 
 void tc_build(Model& m) {
@@ -862,17 +782,8 @@ void tc_build(Model& m) {
         s.b3 = f.conv3.b;
     };
     fc_tc_init();
-    {
-        const char* e = getenv("P2S_FC_FP32");
-        t->fc_on_tc = !(e && e[0] == '1');
-    }
-    auto mk_fc = [&](const Layer& L) {
-        TcFc f;
-        f.L = &L;
-        f.img = fc_tc_supported(L.cout, L.cin) ? fc_tc_pack(L, t->allocs) : nullptr;
-        return f;
-    };
-    auto mk_stn_fc = [&](const Stn& s) { TcStnFc r; r.fc1 = mk_fc(s.fc1); r.fc2 = mk_fc(s.fc2); r.fc3 = mk_fc(s.fc3); return r; };
+    // every FC layer but the QSTN's fc3 (256 -> 4) and fc4 (128 -> 2) runs on the tensor-core FC kernel; fc_tc_pack checks the shape
+    auto mk_stn_fc = [&](const Stn& s) { TcStnFc r; r.fc1 = fc_tc_pack(s.fc1, t->allocs); r.fc2 = fc_tc_pack(s.fc2, t->allocs); return r; };
     if (m.shared_qstn) t->qstn_fc = mk_stn_fc(m.point_stn);
     else if (m.global.has_qstn) t->qstn_fc = mk_stn_fc(m.global.stn1);
     t->stn_fc[0] = mk_stn_fc(m.local.stn2);
@@ -886,10 +797,10 @@ void tc_build(Model& m) {
         t->fold_img[br] = fc_tc_pack_raw(G, 4096, 256, t->allocs);
         t->fold_bias[br] = g0;
     }
-    t->head_fc1[0] = mk_fc(m.fc1_local);
-    t->head_fc1[1] = mk_fc(m.fc1_global);
-    t->head_fc2 = mk_fc(m.fc2);
-    t->head_fc3 = mk_fc(m.fc3);
+    t->head_fc1[0] = fc_tc_pack(m.fc1_local, t->allocs);
+    t->head_fc1[1] = fc_tc_pack(m.fc1_global, t->allocs);
+    t->head_fc2 = fc_tc_pack(m.fc2, t->allocs);
+    t->head_fc3 = fc_tc_pack(m.fc3, t->allocs);
     if (m.shared_qstn) build_stn(t->qstn, m.point_stn, nullptr, nullptr);
     else if (m.global.has_qstn) build_stn(t->qstn, m.global.stn1, nullptr, nullptr);
     build_stn(t->stn[0], m.local.stn2, &m.local.conv0a, &m.local.conv0b);
@@ -933,28 +844,25 @@ static void forward_tc_core(Model& m, const float* patch, const float* sub, cons
     TcWeights& t = *m.tc;
     const int P = m.cfg.points_per_patch, S = m.cfg.sub_sample_size;
     const int64_t Bc_max = 8192;
-    // workspace (floats per query)
-    const size_t per_q = 1024 * 4 + 512 + 256 + 4 + 9 + 4096 * 2 + 1024 + 256 + 128 + 4096 /* 16 KB perq image (hi | lo) */ + 16 +
-                         1024 + 512 + 256 /* A operand images of the FC tails (4 B per element: hi + lo fp16) */;
+    // workspace (floats per query): gmax, f2, q4, R, fmax_l, fmax_g, cat, h4, the 16 KB per-query image (hi | lo) and the
+    // A operand images of the FC tails (4 B per element: hi + lo fp16) for K = 1024, 512, 256
+    const size_t per_q = 1024 + 256 + 4 + 9 + 1024 * 3 + 128 + 4096 + 1024 + 512 + 256;
     float* base = m.ws_net.as<float>(per_q * (size_t)Bc_max + 1024);
     float* pcur = base;
     auto take = [&](size_t n) { float* r = pcur; pcur += (n * (size_t)Bc_max + 63) / 64 * 64; return r; };
-    float* gmax = take(1024); float* g = take(1024); float* f1 = take(512); float* f2 = take(256);
-    float* q4 = take(4); float* R = take(9); float* T = take(4096); float* Tt = take(4096);
-    float* fmax_l = take(1024); float* fmax_g = take(1024); float* cat = take(1024); float* h3 = take(256); float* h4 = take(128);
+    float* gmax = take(1024); float* f2 = take(256); float* q4 = take(4); float* R = take(9);
+    float* fmax_l = take(1024); float* fmax_g = take(1024); float* cat = take(1024); float* h4 = take(128);
     uint8_t* perq = reinterpret_cast<uint8_t*>(take(4096));
-    // A operand images (hi | lo fp16, 4 B per element; Bc_max is a multiple of 128): K = 1024, 512, 256
+    // (Bc_max is a multiple of 128, so every image of Bc_max rows fits its slice)
     uint8_t* imgA = reinterpret_cast<uint8_t*>(take(1024)); uint8_t* imgB = reinterpret_cast<uint8_t*>(take(512)); uint8_t* imgC = reinterpret_cast<uint8_t*>(take(256));
-    const bool fc_tc = t.fc_on_tc || precise;   // the precise path needs the split-precision FC kernel's image output
     // FC tails as a chain of operand images: the raw max features are packed once (bias + ReLU on the way), every layer reads
     // its A operand by bulk copy and writes its output as the next layer's image -- no per-N-tile re-conversion of A
-    auto img_ok = [](const TcStnFc& f) { return f.fc1.img && f.fc2.img; };
     // gmax_raw [Bc,1024] -> relu(+b3) -> fc1 -> fc2; f2 as fp32 rows (out_f2) or as an image in imgC
-    auto stn_tail_img = [&](const Layer& c3, const TcStnFc& f, const float* gmax_raw, int64_t Bc, float* out_f2) {
-        launch_pack_a(gmax_raw, 1024, Bc, 1024, c3.b, true, imgA, st);
-        launch_fc_tc_img(imgA, f.fc1.img, f.fc1.L->b, imgB, 0, Bc, 512, 1024, true, st, 3, 16, 0);
-        if (out_f2) launch_fc_tc_img(imgB, f.fc2.img, f.fc2.L->b, out_f2, 256, Bc, 256, 512, true, st, 0);
-        else launch_fc_tc_img(imgB, f.fc2.img, f.fc2.L->b, imgC, 0, Bc, 256, 512, true, st, 3, 8, 0);
+    auto stn_tail_img = [&](const Stn& s, const TcStnFc& f, const float* gmax_raw, int64_t Bc, float* out_f2) {
+        launch_pack_a(gmax_raw, 1024, Bc, 1024, s.c3.b, true, imgA, st);
+        launch_fc_tc_img(imgA, f.fc1, s.fc1.b, imgB, 0, Bc, 512, 1024, true, st, 3, 16, 0);
+        if (out_f2) launch_fc_tc_img(imgB, f.fc2, s.fc2.b, out_f2, 256, Bc, 256, 512, true, st, 0);
+        else launch_fc_tc_img(imgB, f.fc2, s.fc2.b, imgC, 0, Bc, 256, 512, true, st, 3, 8, 0);
     };
 
     for (int64_t b0 = 0; b0 < B; b0 += Bc_max) {
@@ -963,22 +871,15 @@ static void forward_tc_core(Model& m, const float* patch, const float* sub, cons
         const float* su = sub + b0 * S * 3;
         const float* qu = query + b0 * 3;
         const float* Rq = nullptr;
-        if (m.shared_qstn) {
-            // pass A over cat(patch, sub - q)   (model.py:303,325-327)
-            { StageScope ts("net: pass kernels", st); launch_pass(m, t.qstn, make_seg(pa, P, 0), make_seg(su, S, 1), qu, nullptr, Bc, -1, nullptr, gmax, st, precise); }
+        if (m.shared_qstn || m.global.has_qstn) {
+            // pass A over cat(patch, sub - q) (shared QSTN, model.py:303,325-327) or over the global branch's sub-sample
+            const Stn& qs = m.shared_qstn ? m.point_stn : m.global.stn1;
+            const Seg s0 = m.shared_qstn ? make_seg(pa, P, 0) : make_seg(su, S, 1);
+            const Seg s1 = m.shared_qstn ? make_seg(su, S, 1) : make_seg(nullptr, 0, 0);
+            { StageScope ts("net: pass kernels", st); launch_pass(m, t.qstn, s0, s1, qu, nullptr, Bc, -1, nullptr, gmax, st, precise); }
             { StageScope ts("net: fc tails", st);
-              if (fc_tc && img_ok(t.qstn_fc)) {
-                  stn_tail_img(m.point_stn.c3, t.qstn_fc, gmax, Bc, f2);
-                  run_fc(t.qstn_fc.fc3, f2, 256, q4, 4, Bc, false, false, st);
-              } else fc_tail(m.point_stn.c3, t.qstn_fc, fc_tc, gmax, Bc, g, f1, f2, q4, st); }
-            launch_quat_to_rot(q4, R, Bc, st);
-            Rq = R;
-        } else if (m.global.has_qstn) {
-            launch_pass(m, t.qstn, make_seg(su, S, 1), make_seg(nullptr, 0, 0), qu, nullptr, Bc, -1, nullptr, gmax, st, precise);
-            if (fc_tc && img_ok(t.qstn_fc)) {
-                stn_tail_img(m.global.stn1.c3, t.qstn_fc, gmax, Bc, f2);
-                run_fc(t.qstn_fc.fc3, f2, 256, q4, 4, Bc, false, false, st);
-            } else fc_tail(m.global.stn1.c3, t.qstn_fc, fc_tc, gmax, Bc, g, f1, f2, q4, st);
+              stn_tail_img(qs, t.qstn_fc, gmax, Bc, f2);
+              launch_gemm_nt(f2, 0, 256, qs.fc3.W, 0, qs.fc3.b, q4, 0, 4, (int)Bc, qs.fc3.cout, qs.fc3.cin, 1, false, st); }
             launch_quat_to_rot(q4, R, Bc, st);
             Rq = R;
         }
@@ -988,61 +889,36 @@ static void forward_tc_core(Model& m, const float* patch, const float* sub, cons
             float* fmax = br ? fmax_g : fmax_l;
             // pass B: STN64 -> T
             { StageScope ts("net: pass kernels", st); launch_pass(m, t.stn[br], sg, make_seg(nullptr, 0, 0), qu, Rq, Bc, -1, nullptr, gmax, st, precise); }
-            if (fc_tc) {
-                // fc1, fc2, then the folded last layer writes the per-query fp16 operand images of conv1*(T+I) directly
+            {   // fc1, fc2, then the folded last layer writes the per-query fp16 operand images of conv1*(T+I) directly
                 StageScope ts("net: fc tails", st);
-                if (img_ok(t.stn_fc[br])) {
-                    stn_tail_img(f.stn2.c3, t.stn_fc[br], gmax, Bc, nullptr);
-                    launch_fc_tc_img(imgC, t.fold_img[br], t.fold_bias[br], perq, 0, Bc, 4096, 256, false, st, precise ? 2 : 1);
-                } else {
-                    run_fc(t.stn_fc[br].fc1, gmax, 1024, f1, 512, Bc, true, true, st, f.stn2.c3.b, true);
-                    run_fc(t.stn_fc[br].fc2, f1, 512, f2, 256, Bc, true, true, st);
-                    launch_fc_tc(f2, 256, t.fold_img[br], t.fold_bias[br], reinterpret_cast<float*>(perq), 0, Bc, 4096, 256, false, st, precise ? 2 : 1);
-                }
-            } else {
-                { StageScope ts("net: fc tails", st); fc_tail(f.stn2.c3, t.stn_fc[br], false, gmax, Bc, g, f1, f2, T, st); }
-                // W1' = conv1.W * (T + I) -> per-query fp16 operand images (one fused kernel)
-                { StageScope ts("net: fold W1*T", st); P2S_LAUNCH(fold_w1_kernel, (unsigned)Bc, 256, 0, st, f.conv1.W, T, Bc, perq); }
+                stn_tail_img(f.stn2, t.stn_fc[br], gmax, Bc, nullptr);
+                launch_fc_tc_img(imgC, t.fold_img[br], t.fold_bias[br], perq, 0, Bc, 4096, 256, false, st, precise ? 2 : 1);
             }
-            (void)Tt;
             // pass C: final stack -> max feature (bias, no ReLU: model.py:203,210-212)
             { StageScope ts("net: pass kernels", st); launch_pass(m, t.fin[br], sg, make_seg(nullptr, 0, 0), qu, Rq, Bc, 1, perq, fmax, st, precise); }
         }
-        // max features = raw max + conv3 bias, no ReLU (model.py:203,210-212): added by the first head FC on load, or by a
-        // separate kernel when the features are exported (debug_aux) or the FCs run on the fp32 kernels
-        const bool fuse_b3 = fc_tc && !m.debug_aux && t.head_fc1[0].img && t.head_fc1[1].img;
-        if (!fuse_b3) {
+        // max features = raw max + conv3 bias, no ReLU (model.py:203,210-212): the bias is added while packing fc1's operand image.
+        // cat(local, global) (model.py:335,343,346) is the K = 1024 operand image of fc2: k-steps 0-15 local, 16-31 global
+        StageScope ts_head("net: fc tails", st);
+        uint8_t* imgCat = reinterpret_cast<uint8_t*>(cat);            // [Bc,1024] x 4 B: same footprint as fp32 rows
+        launch_pack_a(fmax_l, 1024, Bc, 1024, m.local.conv3.b, false, imgA, st);
+        launch_fc_tc_img(imgA, t.head_fc1[0], m.fc1_local.b, imgCat, 0, Bc, 512, 1024, true, st, 3, 32, 0);
+        launch_pack_a(fmax_g, 1024, Bc, 1024, m.global.conv3.b, false, imgA, st);
+        launch_fc_tc_img(imgA, t.head_fc1[1], m.fc1_global.b, imgCat, 0, Bc, 512, 1024, true, st, 3, 32, 16);
+        if (m.debug_aux) {      // exported features: the bias is added in place once both images are packed
             launch_bias_act(fmax_l, m.local.conv3.b, Bc, 1024, false, st);
             launch_bias_act(fmax_g, m.global.conv3.b, Bc, 1024, false, st);
+            debug_aux_copy(m, b0, Bc, Rq, fmax_l, fmax_g, st);
         }
-        debug_aux_copy(m, b0, Bc, Rq, fmax_l, fmax_g, st);
-        StageScope ts_head("net: fc tails", st);
-        if (fuse_b3 && t.head_fc2.img && t.head_fc3.img) {
-            // cat(local, global) (model.py:335,343,346) is the K = 1024 operand image of fc2: k-steps 0-15 local, 16-31 global
-            uint8_t* imgCat = reinterpret_cast<uint8_t*>(cat);            // [Bc,1024] x 4 B: same footprint as the fp32 rows
-            launch_pack_a(fmax_l, 1024, Bc, 1024, m.local.conv3.b, false, imgA, st);
-            launch_fc_tc_img(imgA, t.head_fc1[0].img, m.fc1_local.b, imgCat, 0, Bc, 512, 1024, true, st, 3, 32, 0);
-            launch_pack_a(fmax_g, 1024, Bc, 1024, m.global.conv3.b, false, imgA, st);
-            launch_fc_tc_img(imgA, t.head_fc1[1].img, m.fc1_global.b, imgCat, 0, Bc, 512, 1024, true, st, 3, 32, 16);
-            launch_fc_tc_img(imgCat, t.head_fc2.img, m.fc2.b, imgC, 0, Bc, 256, 1024, true, st, 3, 8, 0);
-            launch_fc_tc_img(imgC, t.head_fc3.img, m.fc3.b, h4, 128, Bc, 128, 256, true, st, 0);
-        } else {
-            run_fc(t.head_fc1[0], fmax_l, 1024, cat, 1024, Bc, true, fc_tc, st, fuse_b3 ? m.local.conv3.b : nullptr, false);
-            run_fc(t.head_fc1[1], fmax_g, 1024, cat + 512, 1024, Bc, true, fc_tc, st, fuse_b3 ? m.global.conv3.b : nullptr, false);
-            run_fc(t.head_fc2, cat, 1024, h3, 256, Bc, true, fc_tc, st);
-            run_fc(t.head_fc3, h3, 256, h4, 128, Bc, true, fc_tc, st);
-        }
+        launch_fc_tc_img(imgCat, t.head_fc2, m.fc2.b, imgC, 0, Bc, 256, 1024, true, st, 3, 8, 0);
+        launch_fc_tc_img(imgC, t.head_fc3, m.fc3.b, h4, 128, Bc, 128, 256, true, st, 0);
         launch_gemm_nt(h4, 0, 128, m.fc4.W, 0, m.fc4.b, logits + b0 * 2, 0, 2, (int)Bc, 2, 128, 1, false, st);
     }
 }
 
-// accurate recompute used for the guard band: split-precision tensor-core path (default) or the fp32 FMA path
-// (environment P2S_GUARD_FP32=1)
+// accurate recompute used for the guard band: the split-precision tensor-core path
 void forward_guard(Model& m, const float* patch, const float* sub, const float* query, int64_t B, float* logits, cudaStream_t st) {
-    static int use_fp32 = -1;
-    if (use_fp32 < 0) { const char* e = getenv("P2S_GUARD_FP32"); use_fp32 = (e && e[0] == '1') ? 1 : 0; }
-    if (use_fp32) forward_fp32(m, patch, sub, query, B, logits, st);
-    else forward_tc_core(m, patch, sub, query, B, logits, st, true);
+    forward_tc_core(m, patch, sub, query, B, logits, st, true);
 }
 
 void forward_tc(Model& m, const float* patch, const float* sub, const float* query, int64_t B,

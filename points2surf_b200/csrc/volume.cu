@@ -633,11 +633,7 @@ void sdf_to_volume(const int32_t* lin_idx, const float* sdf, int64_t Q, int res,
     (void)Z0;
     pp.words = (res % 4 == 0) ? 1 : 0;       // aligned 32-bit row loads need word-aligned rows
     pp.fast = (pp.words && sigma <= 5) ? 1 : 0;   // packed biased-byte sums need 2 * sigma^3 <= 255
-    {
-        static int novec = -1;
-        if (novec < 0) { const char* e = getenv("P2S_VOL_NOVEC"); novec = (e && e[0] == '1') ? 1 : 0; }
-        pp.vec = (sigma == 5 && res % 32 == 0 && !novec) ? 1 : 0;   // row-vector path: full tiles, 16-byte aligned rows
-    }
+    pp.vec = (sigma == 5 && res % 32 == 0) ? 1 : 0;   // row-vector path: full tiles, 16-byte aligned rows
     const size_t smem_generic = (size_t)((X0 * Y0 * ZS + 15) & ~15) + (size_t)((X0 * Y0 * TZ + 15) & ~15) + (size_t)X0 * TY * TZ * 2;
     const size_t smem_fast = 4 * ((size_t)X0 * Y0 * (ZS / 4) + (size_t)TX * TY * 8 + (size_t)X0 * Y0 * 8 + (size_t)X0 * TY * 8);
     const size_t smem = pp.fast ? smem_fast : smem_generic;

@@ -173,51 +173,39 @@ def test_subsample_weighted_is_without_replacement_and_matches_reference_law():
     assert freq_gpu[near[:10]].mean() > freq_gpu[near[-10:]].mean() + 0.1
 
 
-_SAMPLER_SCRIPT = r"""
-import sys, numpy as np, torch
-sys.path.insert(0, %r)
-from oracle import p2s_oracle as orc
-from points2surf_b200 import ops, synth
-dev = 'cuda:0'
-cu = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)
-# (a) law on a small cloud: inclusion frequencies vs RandomState.choice(replace=False, p)
-rng = np.random.RandomState(3)
-cloud = rng.uniform(-0.9, 0.9, (40, 3)).astype(np.float32)
-qp = np.array([[0.3, -0.2, 0.1]], np.float32)
-trials = 4000
-ids = ops.subsample(cu(cloud), cu(np.repeat(qp, trials, axis=0)), 10, False, seed=11).cpu().numpy()
-assert all(len(set(r.tolist())) == 10 for r in ids)
-freq = np.bincount(ids.ravel(), minlength=40) / trials
-prob = orc.sub_sample_probabilities(cloud, qp[0])
-rs = np.random.RandomState(5)
-ref = np.stack([rs.choice(40, size=10, replace=False, p=prob) for _ in range(trials)])
-dev_max = np.abs(freq - np.bincount(ref.ravel(), minlength=40) / trials).max()
-assert dev_max < 0.05, dev_max
-# (b) a surface cloud at the benchmark's sizes: distinct ids in range, near points favoured, slabs reproduce the whole
-cloud = synth.make_cloud('sphere', 10000, seed=0)
-q = cloud[:64] * np.float32(0.97)
-a = ops.subsample(cu(cloud), cu(q), 1000, False, seed=7).cpu().numpy()
-assert a.min() >= 0 and a.max() < 10000 and all(len(set(r.tolist())) == 1000 for r in a)
-b = ops.subsample(cu(cloud), cu(q[10:20]), 1000, False, seed=7, query_index_base=10).cpu().numpy()
-assert np.array_equal(np.sort(a[10:20], axis=1), np.sort(b, axis=1))
-d = np.linalg.norm(cloud[a[0]] - q[0], axis=1)
-assert d.mean() < np.linalg.norm(cloud - q[0], axis=1).mean()
-print('sampler ok', dev_max)
-"""
-
-
-@pytest.mark.parametrize('env', [{}, {'P2S_SUBSAMPLE_NOCELLS': '1'}, {'P2S_SUBSAMPLE_CLOCKS': '1'}])
-def test_subsample_weighted_all_three_kernels_realise_the_reference_law(env):
-    # the cell-index sampler (default), the uniform-proposal rejection sampler and the exponential-clock selection are
-    # switched by environment variables that the library reads once per process -> one subprocess per kernel
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    e = dict(os.environ)
-    e.update(env)
-    r = subprocess.run([sys.executable, '-c', _SAMPLER_SCRIPT % root], env=e, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and 'sampler ok' in r.stdout, (r.stdout[-2000:], r.stderr[-2000:])
+# The weighted sampler picks its kernel from the cloud size (N points, S drawn; the shared-memory cache holds 4 B per point,
+# at most 160 KB): the cell index when N >= 2 S and N <= 40 960, the exponential clocks with the cache when N < 2 S and
+# N <= 40 960, the clocks without the cache above 40 960 points.
+@pytest.mark.parametrize('law,surface', [((40, 10), (10000, 1000)), ((40, 25), (1500, 1000)), (None, (50000, 1000))],
+                         ids=['cells', 'clocks-cached', 'clocks-uncached'])
+def test_subsample_weighted_kernels_realise_the_reference_law(law, surface):
+    if law is not None:
+        # law on a small cloud: inclusion frequencies vs RandomState.choice(replace=False, p)
+        n, S = law
+        rng = np.random.RandomState(3)
+        cloud = rng.uniform(-0.9, 0.9, (n, 3)).astype(np.float32)
+        qp = np.array([[0.3, -0.2, 0.1]], np.float32)
+        trials = 4000
+        ids = ops.subsample(cu(cloud), cu(np.repeat(qp, trials, axis=0)), S, False, seed=11).cpu().numpy()
+        assert all(len(set(r.tolist())) == S for r in ids)
+        freq = np.bincount(ids.ravel(), minlength=n) / trials
+        prob = orc.sub_sample_probabilities(cloud, qp[0])
+        rs = np.random.RandomState(5)
+        ref = np.stack([rs.choice(n, size=S, replace=False, p=prob) for _ in range(trials)])
+        dev_max = np.abs(freq - np.bincount(ref.ravel(), minlength=n) / trials).max()
+        assert dev_max < 0.05, dev_max
+        near = np.argsort(np.linalg.norm(cloud - qp[0], axis=1))
+        assert freq[near[:10]].mean() > freq[near[-10:]].mean() + 0.1
+    # a surface cloud: distinct ids in range, near points favoured, slabs reproduce the whole
+    n, S = surface
+    cloud = synth.make_cloud('sphere', n, seed=0)
+    q = cloud[:64] * np.float32(0.97)
+    a = ops.subsample(cu(cloud), cu(q), S, False, seed=7).cpu().numpy()
+    assert a.min() >= 0 and a.max() < n and all(len(set(r.tolist())) == S for r in a)
+    b = ops.subsample(cu(cloud), cu(q[10:20]), S, False, seed=7, query_index_base=10).cpu().numpy()
+    assert np.array_equal(np.sort(a[10:20], axis=1), np.sort(b, axis=1))
+    d = np.linalg.norm(cloud[a[0]] - q[0], axis=1)
+    assert d.mean() < np.linalg.norm(cloud - q[0], axis=1).mean()
 
 
 def test_subsample_requires_enough_points():
@@ -388,6 +376,8 @@ def test_forward_tc_matches_oracle(variant):
     eng = make_engine(sd, variant, precision='tc', guard_band=0.0)
     args = (cu(inp['patch_pts_ps']), cu(inp['pts_sub_sample_ms']), cu(inp['imp_surf_query_point_ms']))
     out, aux = eng.forward_with_aux(*args)
+    # the aux tap observes the production head: the same logits, bit for bit, as a plain forward
+    assert torch.equal(out, eng.forward(*args))
     ref, raux = orc.model_forward(sd, inp['patch_pts_ps'], inp['pts_sub_sample_ms'], inp['imp_surf_query_point_ms'],
                                   v['use_point_stn'], v['shared_transformer'], return_aux=True)
     if 'trans' in raux:
