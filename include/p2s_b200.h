@@ -11,7 +11,8 @@
  *     (thread-local, valid until the next call on the same thread).
  *   - `*_dev` functions take DEVICE pointers on the model's device and enqueue on `stream`
  *     (a cudaStream_t passed as void*; NULL = default stream).  They do not synchronise unless
- *     documented ("sync: count read-back").
+ *     documented ("sync: count read-back").  Functions without a model run on the calling thread's
+ *     current CUDA device, which must be the device of their pointers and of `stream`.
  *   - `*_host` functions take HOST pointers, perform H2D/D2H copies on the model's internal stream
  *     and return after the result is in the host buffer.
  *   - all float data is IEEE fp32, all index data int32, row-major, densely packed.
@@ -70,14 +71,15 @@ int p2s_model_create(const p2s_model_config* cfg, const float* blob_host, size_t
 void p2s_model_destroy(p2s_model* m);
 
 /* Arithmetic of the per-point MLP stacks:
- *   P2S_PRECISION_FP32  CUDA-core fp32 FMA everywhere (accuracy path; also the guard-band recompute path)
+ *   P2S_PRECISION_FP32  CUDA-core fp32 FMA everywhere (accuracy path)
  *   P2S_PRECISION_TC    tcgen05 tensor cores, fp16 operands (11-bit significand, same as the TF32 the
  *                       reference's cuDNN Conv1d uses on Ampere+), fp32 accumulate; queries whose
- *                       |sign logit| < guard_band are recomputed on the fp32 path. */
+ *                       |sign logit| < guard_band are recomputed on the tensor cores in split precision
+ *                       (hi + lo fp16 operands, fp32-level accuracy). */
 #define P2S_PRECISION_FP32 0
 #define P2S_PRECISION_TC 1
 int p2s_model_set_precision(p2s_model* m, int precision, float guard_band);
-/* number of queries the last forward recomputed on the fp32 path (guard band); sync. */
+/* number of queries recomputed in split precision (guard band) since the last call; sync. */
 int p2s_model_last_guard_count(p2s_model* m, int64_t* count);
 
 /* Instrumentation for bench.py's roofline: when enabled, every launch of the dominant kernel (the tensor-core

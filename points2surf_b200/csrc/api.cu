@@ -6,17 +6,46 @@ namespace p2s {
 thread_local std::string g_last_error;
 std::atomic<uint64_t> g_launches{0};
 
+DeviceCtx& device_ctx() {
+    // the device memory of a context is never freed (a thread's exit may come after the CUDA runtime's)
+    static thread_local std::vector<std::unique_ptr<DeviceCtx>> table;
+    int dev = 0;
+    P2S_CUDA(cudaGetDevice(&dev));
+    if ((int)table.size() <= dev) table.resize(dev + 1);
+    if (!table[dev]) {
+        auto c = std::make_unique<DeviceCtx>();
+        c->device = dev;
+        P2S_CUDA(cudaDeviceGetAttribute(&c->sm_count, cudaDevAttrMultiProcessorCount, dev));
+        P2S_CUDA(cudaMalloc(&c->err_flag, sizeof(int)));
+        P2S_CUDA(cudaMemset(c->err_flag, 0, sizeof(int)));
+        table[dev] = std::move(c);
+    }
+    return *table[dev];
+}
+
+void DeviceCtx::set_max_dynamic_smem(const void* fn, int bytes) {
+    for (auto& f : smem_limits) {
+        if (f.first != fn) continue;
+        if (f.second < bytes) {
+            P2S_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+            f.second = bytes;
+        }
+        return;
+    }
+    P2S_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    smem_limits.emplace_back(fn, bytes);
+}
+
 // grid.cu / assemble.cu / volume.cu / mc.cu
 void query_grid(const float* pts, int64_t N, int res, int eps, int32_t* lin_idx, int64_t cap, int64_t* count_host, cudaStream_t st);
 void query_points(const int32_t* lin_idx, int64_t Q, int res, float* out, cudaStream_t st);
 void knn_patch(const float* pts, int64_t N, const float* queries, int64_t Q, int k, int32_t* ids, float* patch, float* radius, cudaStream_t st);
 void ball_patch(const float* pts, int64_t N, const float* queries, int64_t Q, int64_t qbase, int k, double patch_radius, uint64_t seed, int32_t* ids, float* patch, float* radius, int32_t* counts, cudaStream_t st, const int32_t* qidx = nullptr);
-struct CloudIndex;
 bool cloud_index_usable(int64_t N, int S, int mode);
 const CloudIndex* cloud_index_build(const float* pts, int64_t N, cudaStream_t st);
 void subsample(const float* pts, int64_t N, const float* queries, int64_t Q, int64_t qbase, int S, int mode, uint64_t seed, int32_t* out, cudaStream_t st, const int32_t* qidx = nullptr, float* pts_out = nullptr, const CloudIndex* cidx = nullptr);
-void gather_i32(const int32_t* src, const int32_t* idx, int64_t n, int32_t* dst, cudaStream_t st);
-void scatter_f32(const float* src, const int32_t* idx, int64_t n, float* dst, cudaStream_t st);
+void gather_rows(const void* src, const int32_t* rows, int64_t n, int words, void* dst, cudaStream_t st);
+void scatter_rows(const void* src, const int32_t* rows, int64_t n, int words, void* dst, cudaStream_t st);
 void gather_points(const float* pts, const int32_t* ids, int64_t count, float* out, cudaStream_t st);
 int assemble_error_check(cudaStream_t st);
 void sdf_from_logits(const float* logits, const float* radius, int64_t B, float* sdf, cudaStream_t st);
@@ -106,10 +135,38 @@ struct BatchBufs {
 
 }  // namespace
 
-void forward(Model& m, const float* patch, const float* sub, const float* query, int64_t B, float* logits, cudaStream_t st) {
-    if (B <= 0) return;
-    if (m.precision == P2S_PRECISION_TC) forward_tc(m, patch, sub, query, B, logits, st);
+// the network without the guard band
+static void forward_fast(Model& m, const float* patch, const float* sub, const float* query, int64_t B, float* logits, cudaStream_t st) {
+    if (m.precision == P2S_PRECISION_TC) forward_tc(m, patch, sub, query, B, logits, st, false);
     else forward_fp32(m, patch, sub, query, B, logits, st);
+}
+
+// guard band of the tensor-core path: queries whose |sign logit| < guard_band, too close to 0 for fp16-operand arithmetic,
+// are recomputed by the split-precision pass
+static bool guard_on(const Model& m) { return m.precision == P2S_PRECISION_TC && m.guard_band > 0.f; }
+
+static void forward(Model& m, const float* patch, const float* sub, const float* query, int64_t B, float* logits, cudaStream_t st) {
+    if (B <= 0) return;
+    forward_fast(m, patch, sub, query, B, logits, st);
+    if (!guard_on(m)) return;
+    StageScope ts_guard("net: guard-band split-precision recompute", st);
+    int32_t* list = m.ws_guard.as<int32_t>((size_t)B + 64);
+    int* count = reinterpret_cast<int*>(list + B);
+    P2S_CUDA(cudaMemsetAsync(count, 0, sizeof(int), st));
+    guard_flag(logits, B, m.guard_band, 0, list, count, B, st);
+    int n = 0;
+    P2S_CUDA(cudaMemcpyAsync(&n, count, sizeof(int), cudaMemcpyDeviceToHost, st));
+    P2S_CUDA(cudaStreamSynchronize(st));
+    m.last_guard_count += n;
+    if (n == 0) return;
+    const int rowp = m.cfg.points_per_patch * 3, rows = m.cfg.sub_sample_size * 3;
+    float* gp = m.ws_misc.as<float>((size_t)n * (rowp + rows + 3 + 2) + 64);
+    float* gs = gp + (size_t)n * rowp; float* gq = gs + (size_t)n * rows; float* gl = gq + ((size_t)n * 3 + 3) / 4 * 4;
+    gather_rows(patch, list, n, rowp, gp, st);
+    gather_rows(sub, list, n, rows, gs, st);
+    gather_rows(query, list, n, 3, gq, st);
+    forward_tc(m, gp, gs, gq, n, gl, st, true);
+    scatter_rows(gl, list, n, 2, logits, st);
 }
 
 static void reconstruct(Model& m, const p2s_recon_config& rc, const float* pts, int64_t N, int64_t first_query,
@@ -119,7 +176,7 @@ static void reconstruct(Model& m, const p2s_recon_config& rc, const float* pts, 
     const int P = m.cfg.points_per_patch, S = m.cfg.sub_sample_size;
     int64_t Qall = 0;
     const int64_t vox = (int64_t)rc.res * rc.res * rc.res;
-    int32_t* all_idx = m.ws_misc.as<int32_t>((size_t)vox + 2 * 16384 + 64);   // worst case candidate list (+ guard scratch behind it)
+    int32_t* all_idx = m.ws_misc.as<int32_t>((size_t)vox + 64);   // worst case candidate list
     { StageScope t("grid", st); query_grid(pts, N, rc.res, rc.eps, all_idx, vox, &Qall, st); }
     if (first_query < 0) first_query = 0;
     if (first_query > Qall) first_query = Qall;
@@ -138,16 +195,20 @@ static void reconstruct(Model& m, const p2s_recon_config& rc, const float* pts, 
     auto take = [&](size_t n) { float* r = p; p += (n * (size_t)batch + 3) / 4 * 4; return r; };
     b.qpts = take(3); b.patch = take((size_t)P * 3); b.radius = take(1); b.sub = take((size_t)S * 3); b.logits = take(2);
     b.sub_ids = reinterpret_cast<int32_t*>(take((size_t)S));
-    // guard band of the tensor-core path: flagged queries are collected over the whole slab and recomputed on the
-    // fp32 path in one batch at the end (large GEMMs instead of ~80-query slivers per batch)
-    const bool defer_guard = (m.precision == P2S_PRECISION_TC) && (m.guard_band > 0.f);
+    // guard band: flagged queries are collected over the whole slab and recomputed at the end, in batches of the same
+    // size (large GEMMs instead of ~80-query slivers per batch).  ws_guard holds the slab-relative indices of the flagged
+    // queries [Q], their voxel indices and SDF values of one recompute batch [batch each], and their count.
+    const bool guard = guard_on(m);
     int32_t* glist = nullptr;
+    int32_t* glin = nullptr;
+    float* gsdf = nullptr;
     int* gcount = nullptr;
-    if (defer_guard) {
-        glist = m.ws_guard.as<int32_t>((size_t)Q + 64);
-        gcount = reinterpret_cast<int*>(glist + Q);
+    if (guard) {
+        glist = m.ws_guard.as<int32_t>((size_t)Q + 2 * (size_t)batch + 1);
+        glin = glist + Q;
+        gsdf = reinterpret_cast<float*>(glin + batch);
+        gcount = reinterpret_cast<int*>(gsdf + batch);
         P2S_CUDA(cudaMemsetAsync(gcount, 0, sizeof(int), st));
-        m.guard_list = glist; m.guard_list_count = gcount; m.guard_list_cap = Q;
     }
     // cell index of the cloud for the weighted sub-sampler: once per shape
     const CloudIndex* cidx = cloud_index_usable(N, S, rc.subsample_mode) ? cloud_index_build(pts, N, st) : nullptr;
@@ -160,36 +221,28 @@ static void reconstruct(Model& m, const p2s_recon_config& rc, const float* pts, 
         { StageScope t("assemble: subsample+gather", st);
           subsample(pts, N, b.qpts, n, qbase, S, rc.subsample_mode, rc.seed, b.sub_ids, st, qidx, b.sub, cidx); }
     };
-    try {
-        for (int64_t q0 = 0; q0 < Q; q0 += batch) {
-            const int64_t n = (Q - q0 < batch) ? (Q - q0) : batch;
-            assemble(lin_idx + q0, n, first_query + q0, nullptr);
-            m.guard_base = q0;
-            forward(m, b.patch, b.sub, b.qpts, n, b.logits, st);
-            sdf_from_logits(b.logits, fixed_radius ? nullptr : b.radius, n, sdf + q0, st);
+    for (int64_t q0 = 0; q0 < Q; q0 += batch) {
+        const int64_t n = (Q - q0 < batch) ? (Q - q0) : batch;
+        assemble(lin_idx + q0, n, first_query + q0, nullptr);
+        forward_fast(m, b.patch, b.sub, b.qpts, n, b.logits, st);
+        if (guard) guard_flag(b.logits, n, m.guard_band, q0, glist, gcount, Q, st);
+        sdf_from_logits(b.logits, fixed_radius ? nullptr : b.radius, n, sdf + q0, st);
+    }
+    if (guard) {
+        int ng = 0;
+        P2S_CUDA(cudaMemcpyAsync(&ng, gcount, sizeof(int), cudaMemcpyDeviceToHost, st));
+        P2S_CUDA(cudaStreamSynchronize(st));
+        if (ng > Q) ng = (int)Q;
+        m.last_guard_count += ng;
+        StageScope tg("net: guard-band split-precision recompute", st);
+        for (int64_t g0 = 0; g0 < ng; g0 += batch) {
+            const int64_t n = (ng - g0 < batch) ? (ng - g0) : batch;
+            gather_rows(lin_idx, glist + g0, n, 1, glin, st);
+            assemble(glin, n, first_query, glist + g0);
+            forward_tc(m, b.patch, b.sub, b.qpts, n, b.logits, st, true);
+            sdf_from_logits(b.logits, fixed_radius ? nullptr : b.radius, n, gsdf, st);
+            scatter_rows(gsdf, glist + g0, n, 1, sdf, st);
         }
-        if (defer_guard) {
-            m.guard_list = nullptr;
-            int ng = 0;
-            P2S_CUDA(cudaMemcpyAsync(&ng, gcount, sizeof(int), cudaMemcpyDeviceToHost, st));
-            P2S_CUDA(cudaStreamSynchronize(st));
-            if (ng > Q) ng = (int)Q;
-            m.last_guard_count += ng;
-            StageScope tg("net: guard-band fp32 recompute", st);
-            int32_t* glin = reinterpret_cast<int32_t*>(m.ws_misc.as<float>((size_t)vox + (size_t)batch * 2 + 64) + vox);   // behind all_idx
-            float* gsdf = reinterpret_cast<float*>(glin + batch);
-            for (int64_t g0 = 0; g0 < ng; g0 += batch) {
-                const int64_t n = (ng - g0 < batch) ? (ng - g0) : batch;
-                gather_i32(lin_idx, glist + g0, n, glin, st);
-                assemble(glin, n, first_query, glist + g0);
-                forward_guard(m, b.patch, b.sub, b.qpts, n, b.logits, st);
-                sdf_from_logits(b.logits, fixed_radius ? nullptr : b.radius, n, gsdf, st);
-                scatter_f32(gsdf, glist + g0, n, sdf, st);
-            }
-        }
-    } catch (...) {
-        m.guard_list = nullptr;
-        throw;
     }
     int err = assemble_error_check(st);
     P2S_CHECK(err == 0, "degenerate cloud: more than 512 points tie at a selection boundary");
@@ -231,8 +284,6 @@ int p2s_model_create(const p2s_model_config* cfg, const float* blob_host, size_t
         P2S_CUDA(cudaMalloc(&m->blob, n_floats * sizeof(float)));
         P2S_CUDA(cudaMemcpy(m->blob, blob_host, n_floats * sizeof(float), cudaMemcpyHostToDevice));
         P2S_CUDA(cudaStreamCreateWithFlags(&m->own_stream, cudaStreamNonBlocking));
-        P2S_CUDA(cudaMalloc(&m->guard_count_dev, sizeof(int64_t)));
-        P2S_CUDA(cudaMemset(m->guard_count_dev, 0, sizeof(int64_t)));
         BlobCursor c{m->blob, n_floats};
         const int net = cfg->net_size;
         m->shared_qstn = cfg->use_point_stn && cfg->shared_transformer;
@@ -257,7 +308,6 @@ void p2s_model_destroy(p2s_model* mm) {
     StageTimer::report();
     tc_destroy(*m);
     if (m->blob) cudaFree(m->blob);
-    if (m->guard_count_dev) cudaFree(m->guard_count_dev);
     m->ws_net.release(); m->ws_io.release(); m->ws_misc.release(); m->ws_guard.release(); m->ws_host.release();
     if (m->own_stream) cudaStreamDestroy(m->own_stream);
     delete m;

@@ -12,15 +12,6 @@
 
 namespace p2s {
 
-// per-cloud cell index of the weighted sub-sampler (device pointers; see cloud_index_build)
-struct CloudIndex {
-    const float* meta;      // [6] bounding-box low corner, cells per unit length
-    const float* spts;      // [N,3] points in cell order
-    const int32_t* perm;    // [N]   original id of sorted point i
-    const int32_t* start;   // [C+1] first sorted point of each cell
-    const float* cbox;      // [C,6] tight bounding box of each cell's points
-};
-
 namespace {
 
 constexpr int kThreads = 256;
@@ -884,20 +875,11 @@ __global__ void gather_points_kernel(const float* __restrict__ pts, const int32_
 
 }  // namespace
 
-static int* err_flag_dev() {
-    static thread_local int* flag = nullptr;
-    if (!flag) {
-        P2S_CUDA(cudaMalloc(&flag, sizeof(int)));
-        P2S_CUDA(cudaMemset(flag, 0, sizeof(int)));
-    }
-    return flag;
-}
-
 void gather_points(const float* pts, const int32_t* ids, int64_t count, float* out, cudaStream_t st);
 
 int assemble_error_check(cudaStream_t st) {  // sync; returns and clears the device error flag
     int h = 0;
-    int* f = err_flag_dev();
+    int* f = device_ctx().err_flag;
     P2S_CUDA(cudaMemcpyAsync(&h, f, sizeof(int), cudaMemcpyDeviceToHost, st));
     P2S_CUDA(cudaStreamSynchronize(st));
     if (h) P2S_CUDA(cudaMemsetAsync(f, 0, sizeof(int), st));
@@ -913,21 +895,19 @@ void knn_patch(const float* pts, int64_t N, const float* queries, int64_t Q, int
     // Run length: with 8 queries per CTA a batch of 8 192 queries is 1 024 CTAs = 1.4 waves of the 740 co-resident CTAs, i.e.
     // two waves with the second 38 % full.  Lengthen the runs so that the whole batch is ONE wave (longer runs also amortise
     // the histogram selection of a run's first query better).
-    static thread_local int slots_small = 0, slots_big = 0;
-    if (!slots_small) {
-        int dev = 0, sms = 0, a = 0, b = 0;
-        P2S_CUDA(cudaGetDevice(&dev));
-        P2S_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    DeviceCtx& ctx = device_ctx();
+    if (!ctx.knn_slots_small) {
+        int a = 0, b = 0;
         P2S_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, knn_patch_kernel<kCap>, kThreads, 0));
         P2S_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, knn_patch_kernel<kCapBig>, kThreads, 0));
-        slots_small = sms * (a > 0 ? a : 1); slots_big = sms * (b > 0 ? b : 1);
+        ctx.knn_slots_small = ctx.sm_count * (a > 0 ? a : 1); ctx.knn_slots_big = ctx.sm_count * (b > 0 ? b : 1);
     }
-    const int slots = k <= 512 ? slots_small : slots_big;
+    const int slots = k <= 512 ? ctx.knn_slots_small : ctx.knn_slots_big;
     int run = (int)cdiv(Q, slots);
     if (run < kRun) run = kRun;
     if (run > 64) run = 64;
-    if (k <= 512) P2S_LAUNCH(knn_patch_kernel<kCap>, (unsigned)cdiv(Q, run), kThreads, 0, st, pts, (int)N, queries, Q, k, ids, patch, radius, err_flag_dev(), run);
-    else P2S_LAUNCH(knn_patch_kernel<kCapBig>, (unsigned)cdiv(Q, run), kThreads, 0, st, pts, (int)N, queries, Q, k, ids, patch, radius, err_flag_dev(), run);
+    if (k <= 512) P2S_LAUNCH(knn_patch_kernel<kCap>, (unsigned)cdiv(Q, run), kThreads, 0, st, pts, (int)N, queries, Q, k, ids, patch, radius, ctx.err_flag, run);
+    else P2S_LAUNCH(knn_patch_kernel<kCapBig>, (unsigned)cdiv(Q, run), kThreads, 0, st, pts, (int)N, queries, Q, k, ids, patch, radius, ctx.err_flag, run);
 }
 
 // the Philox stream of query q is keyed by qbase + (qidx ? qidx[q] : q), like the sub-sampler's
@@ -938,12 +918,12 @@ void ball_patch(const float* pts, int64_t N, const float* queries, int64_t Q, in
     P2S_CHECK(N >= 1 && N < (1 << 30), "bad cloud size");
     if (Q <= 0) return;
     P2S_LAUNCH(ball_patch_kernel, (unsigned)Q, kThreads, 0, st, pts, (int)N, queries, qbase, qidx, k, patch_radius * patch_radius,
-               (float)patch_radius, seed, ids, patch, radius, counts, err_flag_dev());
+               (float)patch_radius, seed, ids, patch, radius, counts, device_ctx().err_flag);
 }
 
 // Cell index of a cloud for the weighted sub-sampler: bounding box -> cell keys -> stable radix sort (points of a cell keep
-// their id order, so the result is deterministic) -> per-cell ranges, sorted points, tight boxes.  The index lives in a
-// thread-local workspace and is valid until the next call on this thread (stream order).
+// their id order, so the result is deterministic) -> per-cell ranges, sorted points, tight boxes.  The index lives in the
+// device context and is valid until the next call on this thread and device (stream order).
 constexpr size_t kSubsampleCacheBytes = 160 * 1024;   // dynamic shared memory of the cell and cached clock kernels: 4 B per point
 
 bool cloud_index_usable(int64_t N, int S, int mode) {
@@ -951,8 +931,7 @@ bool cloud_index_usable(int64_t N, int S, int mode) {
 }
 
 const CloudIndex* cloud_index_build(const float* pts, int64_t N, cudaStream_t st) {
-    static thread_local DevBuf ws;
-    static thread_local CloudIndex ci;
+    DeviceCtx& ctx = device_ctx();
     const int n = (int)N;
     size_t cub_bytes = 0;
     P2S_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, (const uint32_t*)nullptr, (uint32_t*)nullptr, (const int32_t*)nullptr, (int32_t*)nullptr, n, 0, 11, st));
@@ -967,7 +946,7 @@ const CloudIndex* cloud_index_build(const float* pts, int64_t N, cudaStream_t st
     const size_t o_spts = off; off += al((size_t)n * 12);
     const size_t o_cbox = off; off += al((size_t)kCC * 24);
     const size_t o_cub = off; off += al(cub_bytes);
-    uint8_t* b = (uint8_t*)ws.get(off);
+    uint8_t* b = (uint8_t*)ctx.cloud_ws.get(off);
     float* meta = (float*)(b + o_meta);
     uint32_t* key = (uint32_t*)(b + o_key); int32_t* val = (int32_t*)(b + o_val);
     uint32_t* key_s = (uint32_t*)(b + o_keys); int32_t* perm = (int32_t*)(b + o_perm);
@@ -976,6 +955,7 @@ const CloudIndex* cloud_index_build(const float* pts, int64_t N, cudaStream_t st
     P2S_CUDA(cub::DeviceRadixSort::SortPairs(b + o_cub, cub_bytes, key, key_s, val, perm, n, 0, 11, st));    // kCC = 1728 < 2^11
     g_launches.fetch_add(3, std::memory_order_relaxed);
     P2S_LAUNCH(ci_finish_kernel, (unsigned)cdiv(kCC + 1, 128), 128, 0, st, pts, n, key_s, perm, (int32_t*)(b + o_start), (float*)(b + o_spts), (float*)(b + o_cbox));
+    CloudIndex& ci = ctx.cloud_index;
     ci.meta = meta; ci.spts = (const float*)(b + o_spts); ci.perm = perm; ci.start = (const int32_t*)(b + o_start); ci.cbox = (const float*)(b + o_cbox);
     return &ci;
 }
@@ -994,21 +974,18 @@ void subsample(const float* pts, int64_t N, const float* queries, int64_t Q, int
         P2S_LAUNCH(subsample_uniform_kernel, (unsigned)cdiv(threads, 256), 256, 0, st, (int)N, Q, qbase, qidx, S, seed, out);
     } else if (mode == P2S_SUBSAMPLE_WEIGHTED) {
         const size_t cache_bytes = (size_t)N * sizeof(float);
-        static thread_local bool attr_set = false;
-        if (!attr_set) {
-            P2S_CUDA(cudaFuncSetAttribute(subsample_cells_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSubsampleCacheBytes));
-            P2S_CUDA(cudaFuncSetAttribute(subsample_weighted_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSubsampleCacheBytes));
-            attr_set = true;
-        }
+        DeviceCtx& ctx = device_ctx();
         if (cloud_index_usable(N, S, mode)) {
             // rejection over the cell index: cheap when at most half of the cloud is drawn
             if (!cidx) cidx = cloud_index_build(pts, N, st);
-            P2S_LAUNCH(subsample_cells_kernel, (unsigned)Q, kThreads, cache_bytes, st, *cidx, (int)N, queries, qbase, qidx, S, seed, out, pts_out, err_flag_dev());
+            ctx.set_max_dynamic_smem((const void*)subsample_cells_kernel, (int)kSubsampleCacheBytes);
+            P2S_LAUNCH(subsample_cells_kernel, (unsigned)Q, kThreads, cache_bytes, st, *cidx, (int)N, queries, qbase, qidx, S, seed, out, pts_out, ctx.err_flag);
             gathered = true;
         } else if (cache_bytes <= kSubsampleCacheBytes) {
-            P2S_LAUNCH(subsample_weighted_kernel<true>, (unsigned)Q, kThreads, cache_bytes, st, pts, (int)N, queries, qbase, qidx, S, seed, out, err_flag_dev());
+            ctx.set_max_dynamic_smem((const void*)subsample_weighted_kernel<true>, (int)kSubsampleCacheBytes);
+            P2S_LAUNCH(subsample_weighted_kernel<true>, (unsigned)Q, kThreads, cache_bytes, st, pts, (int)N, queries, qbase, qidx, S, seed, out, ctx.err_flag);
         } else {
-            P2S_LAUNCH(subsample_weighted_kernel<false>, (unsigned)Q, kThreads, 0, st, pts, (int)N, queries, qbase, qidx, S, seed, out, err_flag_dev());
+            P2S_LAUNCH(subsample_weighted_kernel<false>, (unsigned)Q, kThreads, 0, st, pts, (int)N, queries, qbase, qidx, S, seed, out, ctx.err_flag);
         }
     } else {
         throw Error("unknown sub-sample mode");
@@ -1016,19 +993,24 @@ void subsample(const float* pts, int64_t N, const float* queries, int64_t Q, int
     if (pts_out && !gathered) gather_points(pts, out, Q * S, pts_out, st);
 }
 
-__global__ void gather_i32_kernel(const int32_t* __restrict__ src, const int32_t* __restrict__ idx, int64_t n, int32_t* __restrict__ dst) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) dst[i] = src[idx[i]];
+// rows of `words` 32-bit words: dst[i] = src[rows[i]] (gather), dst[rows[i]] = src[i] (scatter), for i < n
+__global__ void gather_rows_kernel(const uint32_t* __restrict__ src, const int32_t* __restrict__ rows, int64_t n, int words, uint32_t* __restrict__ dst) {
+    int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n * words) return;
+    const int64_t i = e / words;
+    dst[e] = src[(int64_t)rows[i] * words + (e - i * words)];
 }
-__global__ void scatter_f32_kernel(const float* __restrict__ src, const int32_t* __restrict__ idx, int64_t n, float* __restrict__ dst) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) dst[idx[i]] = src[i];
+__global__ void scatter_rows_kernel(const uint32_t* __restrict__ src, const int32_t* __restrict__ rows, int64_t n, int words, uint32_t* __restrict__ dst) {
+    int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n * words) return;
+    const int64_t i = e / words;
+    dst[(int64_t)rows[i] * words + (e - i * words)] = src[e];
 }
-void gather_i32(const int32_t* src, const int32_t* idx, int64_t n, int32_t* dst, cudaStream_t st) {
-    if (n > 0) P2S_LAUNCH(gather_i32_kernel, (unsigned)cdiv(n, 256), 256, 0, st, src, idx, n, dst);
+void gather_rows(const void* src, const int32_t* rows, int64_t n, int words, void* dst, cudaStream_t st) {
+    if (n > 0) P2S_LAUNCH(gather_rows_kernel, (unsigned)cdiv(n * words, 256), 256, 0, st, (const uint32_t*)src, rows, n, words, (uint32_t*)dst);
 }
-void scatter_f32(const float* src, const int32_t* idx, int64_t n, float* dst, cudaStream_t st) {
-    if (n > 0) P2S_LAUNCH(scatter_f32_kernel, (unsigned)cdiv(n, 256), 256, 0, st, src, idx, n, dst);
+void scatter_rows(const void* src, const int32_t* rows, int64_t n, int words, void* dst, cudaStream_t st) {
+    if (n > 0) P2S_LAUNCH(scatter_rows_kernel, (unsigned)cdiv(n * words, 256), 256, 0, st, (const uint32_t*)src, rows, n, words, (uint32_t*)dst);
 }
 
 void gather_points(const float* pts, const int32_t* ids, int64_t count, float* out, cudaStream_t st) {

@@ -8,6 +8,8 @@
 #include <string>
 #include <stdexcept>
 #include <atomic>
+#include <memory>
+#include <utility>
 #include <vector>
 
 #include "../../include/p2s_b200.h"
@@ -98,6 +100,40 @@ struct DevBuf {
         bytes = 0;
     }
 };
+
+// Cell index of a cloud for the weighted sub-sampler (assemble.cu): device pointers into DeviceCtx::cloud_ws
+struct CloudIndex {
+    const float* meta;      // [6] bounding-box low corner, cells per unit length
+    const float* spts;      // [N,3] points in cell order
+    const int32_t* perm;    // [N]   original id of sorted point i
+    const int32_t* start;   // [C+1] first sorted point of each cell
+    const float* cbox;      // [C,6] tight bounding box of each cell's points
+};
+
+// Host-side state of the library for one CUDA device, one context per calling thread and device (device_ctx()).
+// Device memory and kernel attributes belong to one device, so a launcher takes them from the context of the device it
+// launches on; per thread, so that two threads never share scratch.  Two streams of one thread do share it: calls that
+// use the same scratch on two streams must be ordered by the caller.
+struct DeviceCtx {
+    int device = 0;
+    int sm_count = 0;
+    int* err_flag = nullptr;                      // device int: selection failure of kNN / ball query / sub-sample
+    int knn_slots_small = 0, knn_slots_big = 0;   // co-resident CTAs of the two kNN kernels (0 = not yet queried)
+    DevBuf grid_ws;                               // candidate grid (grid.cu)
+    DevBuf vol_ws;                                // sign propagation (volume.cu)
+    DevBuf mc_ws;                                 // marching cubes (mc.cu)
+    DevBuf mesh_area, mesh_cum, mesh_cub, mesh_best, mesh_red;   // mesh sampling and metric (meshdist.cu)
+    DevBuf cloud_ws;                              // cell index of the last cloud (assemble.cu) ...
+    CloudIndex cloud_index{};                     // ... and its pointers, valid until the next cloud_index_build
+    DevBuf train_wimg, train_zero_bias;           // weight image and 4096 zeros of the training GEMMs (fc_tc.cu)
+    DevBuf wait_stats;                            // P2S_TC_WAITSTATS counters (net_tc.cu)
+    std::vector<std::pair<const void*, int>> smem_limits;   // dynamic shared-memory limits raised so far
+
+    // raises the dynamic shared-memory limit of kernel `fn` to `bytes` unless this device already allows that much
+    void set_max_dynamic_smem(const void* fn, int bytes);
+};
+// the context of the calling thread's current CUDA device, created on first use
+DeviceCtx& device_ctx();
 
 // ---- Philox4x32-10 (Salmon et al. 2011), counter-based: (key, counter) -> 4 x u32 ----
 __host__ __device__ inline void philox4x32_10(uint32_t k0, uint32_t k1, uint32_t c0, uint32_t c1,

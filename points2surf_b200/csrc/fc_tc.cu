@@ -268,14 +268,6 @@ bool fc_tc_supported(int N, int K) { return (N % 128 == 0) && (K % kBK == 0) && 
 
 uint8_t* fc_tc_pack(const Layer& L, std::vector<void*>& allocs) { return fc_tc_pack_raw(L.W, L.cout, L.cin, allocs); }
 
-void fc_tc_init() {
-    static bool done = false;
-    if (!done) {
-        P2S_CUDA(cudaFuncSetAttribute(fc_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFcSmem));
-        done = true;
-    }
-}
-
 // A as fp32 rows, C as fp32 rows; N may end in a partial 128-column tile (N % 4 == 0)
 void launch_fc_tc(const float* A, int lda, const uint8_t* Wimg, const float* bias, float* C, int ldc,
                   int64_t M, int N, int K, bool relu, cudaStream_t st) {
@@ -283,6 +275,7 @@ void launch_fc_tc(const float* A, int lda, const uint8_t* Wimg, const float* bia
     P2S_CHECK(N % 4 == 0 && N >= 64 && K % kBK == 0 && K >= kBK && lda % 4 == 0 && ldc % 4 == 0, "bad FC shape for the tensor-core kernel");
     P2S_CHECK(cdiv(M, 128) <= 65535, "too many rows for one launch");
     dim3 grid((unsigned)cdiv(N, 128), (unsigned)cdiv(M, 128), 1);
+    device_ctx().set_max_dynamic_smem((const void*)fc_tc_kernel, (int)kFcSmem);
     P2S_LAUNCH(fc_tc_kernel, grid, 160, kFcSmem, st, A, lda, Wimg, bias, C, ldc, (int)M, N, K, relu ? 1 : 0, 0, (const uint8_t*)nullptr, 0, 0);
 }
 
@@ -302,6 +295,7 @@ void launch_fc_tc_img(const uint8_t* Aimg, const uint8_t* Wimg, const float* bia
               "bad FC shape for the tensor-core kernel (operand-image mode)");
     P2S_CHECK(cdiv(M, 128) <= 65535, "too many rows for one launch");
     dim3 grid((unsigned)(N / 128), (unsigned)cdiv(M, 128), 1);
+    device_ctx().set_max_dynamic_smem((const void*)fc_tc_kernel, (int)kFcSmem);
     P2S_LAUNCH(fc_tc_kernel, grid, 160, kFcSmem, st, (const float*)nullptr, 0, Wimg, bias, reinterpret_cast<float*>(C), ldc, (int)M, N, K, relu ? 1 : 0,
                out_mode, Aimg, out_kt_total, out_kt_off);
 }
@@ -325,17 +319,13 @@ bool gemm_nt_tc_ok(const float* A, int lda, const float* C, int ldc, int64_t M, 
 
 void launch_gemm_nt_tc(const float* A, int lda, const float* W, const float* bias, float* C, int ldc, int64_t M, int N,
                        int K, bool relu, cudaStream_t st) {
-    static thread_local DevBuf img, zeros;
-    static thread_local bool zeroed = false;
-    fc_tc_init();
+    DeviceCtx& ctx = device_ctx();
     const int Npad = (int)(cdiv(N, 128) * 128);
-    uint8_t* wimg = reinterpret_cast<uint8_t*>(img.get((size_t)Npad * K * 4));
+    uint8_t* wimg = reinterpret_cast<uint8_t*>(ctx.train_wimg.get((size_t)Npad * K * 4));
     if (!bias) {
-        float* z = zeros.as<float>(4096);
-        if (!zeroed) {
-            P2S_CUDA(cudaMemsetAsync(z, 0, 4096 * sizeof(float), st));
-            zeroed = true;
-        }
+        const bool fresh = !ctx.train_zero_bias.p;
+        float* z = ctx.train_zero_bias.as<float>(4096);
+        if (fresh) P2S_CUDA(cudaMemsetAsync(z, 0, 4096 * sizeof(float), st));
         bias = z;
     }
     P2S_LAUNCH(pack_fc_pad_kernel, (unsigned)cdiv((int64_t)Npad * K, 256), 256, 0, st, W, N, Npad, K, wimg);

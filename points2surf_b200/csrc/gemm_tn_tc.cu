@@ -158,16 +158,10 @@ bool gemm_tn_tc_ok(const float* A, int lda, const float* B, int ldb, int64_t M, 
 // C must already hold the values the product is added to (zeros or a running gradient)
 void launch_gemm_tn_tc(const float* A, int lda, const float* B, int ldb, float* C, int ldc, int64_t M, int N, int K,
                        cudaStream_t st) {
-    static bool attr = false;
-    if (!attr) {
-        P2S_CUDA(cudaFuncSetAttribute(gemm_tn_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmem));
-        attr = true;
-    }
-    int dev = 0, sms = 148;
-    P2S_CUDA(cudaGetDevice(&dev));
-    P2S_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    DeviceCtx& ctx = device_ctx();
+    ctx.set_max_dynamic_smem((const void*)gemm_tn_tc_kernel, (int)kSmem);
     const int64_t tiles = cdiv(N, 128) * cdiv(K, 128);
-    int64_t splits = std::max<int64_t>(1, cdiv(2 * (int64_t)sms, tiles));
+    int64_t splits = std::max<int64_t>(1, cdiv(2 * (int64_t)ctx.sm_count, tiles));
     splits = std::min<int64_t>(splits, cdiv(M, 1024));
     splits = std::min<int64_t>(splits, 65535);
     int64_t rows = cdiv(cdiv(M, splits), kBM) * kBM;

@@ -65,8 +65,6 @@ __global__ void query_points_kernel(const int32_t* __restrict__ lin, int64_t Q, 
     out[i * 3 + 2] = (float)(((double)iz + 0.5) / (double)res * 2.0 - 1.0);
 }
 
-static thread_local DevBuf t_grid_ws;
-
 void query_grid(const float* pts, int64_t N, int res, int eps, int32_t* lin_idx, int64_t cap,
                 int64_t* count_host, cudaStream_t st) {
     P2S_CHECK(res >= 2 && res <= 1024, "grid resolution out of range");
@@ -80,7 +78,7 @@ void query_grid(const float* pts, int64_t N, int res, int eps, int32_t* lin_idx,
     off_sel = (off_sel + 255) / 256 * 256;
     size_t off_num = off_sel + (size_t)vox * 4;
     size_t off_cub = off_num + 256;
-    uint8_t* base = (uint8_t*)t_grid_ws.get(off_cub + cub_bytes);
+    uint8_t* base = (uint8_t*)device_ctx().grid_ws.get(off_cub + cub_bytes);
     uint8_t* occ = base;
     uint8_t* flag = base + off_flag;
     int32_t* sel = (int32_t*)(base + off_sel);

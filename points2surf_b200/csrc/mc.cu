@@ -140,8 +140,6 @@ __global__ void mc_flip_kernel(int32_t* __restrict__ faces, int64_t F, const dou
     faces[i * 3 + 2] = t;
 }
 
-thread_local DevBuf t_mc_ws;
-
 }  // namespace
 
 void marching_cubes(const float* vol, int R, float level, float* verts, int64_t vcap, int32_t* faces, int64_t fcap,
@@ -157,7 +155,7 @@ void marching_cubes(const float* vol, int R, float level, float* verts, int64_t 
     auto al = [](size_t x) { return (x + 255) / 256 * 256; };
     size_t off_flags = 256, off_vid = off_flags + al(E), off_cnt = off_vid + al(E * 4), off_offs = off_cnt + al(C),
            off_cub = off_offs + al(C * 4);
-    uint8_t* base = (uint8_t*)t_mc_ws.get(off_cub + cub_bytes);
+    uint8_t* base = (uint8_t*)device_ctx().mc_ws.get(off_cub + cub_bytes);
     double* acc = (double*)base;
     uint8_t* flags = base + off_flags;
     int32_t* vid = (int32_t*)(base + off_vid);

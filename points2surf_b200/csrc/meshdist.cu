@@ -130,25 +130,14 @@ nn_finalize_kernel(const unsigned long long* __restrict__ best, int64_t na, floa
     }
 }
 
-struct Scratch {
-    DevBuf area, cum, cub_tmp, best, red;
-};
-Scratch& scratch() {
-    static thread_local Scratch s;
-    return s;
-}
-
 void nn_core(const float* a, int64_t na, const float* b, int64_t nb, float* dist, int32_t* idx, double* sum_out,
              unsigned int* max_out, cudaStream_t st) {
-    auto& sc = scratch();
-    unsigned long long* best = sc.best.as<unsigned long long>((size_t)na);
+    DeviceCtx& ctx = device_ctx();
+    unsigned long long* best = ctx.mesh_best.as<unsigned long long>((size_t)na);
     P2S_LAUNCH(nn_init_kernel, (unsigned)cdiv(na, 256), 256, 0, st, best, na);
-    int dev = 0, sms = 148;
-    P2S_CUDA(cudaGetDevice(&dev));
-    P2S_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     int64_t gx = cdiv(na, kNnThreads);
     int64_t max_slabs = cdiv(nb, kNnTile);
-    int64_t slabs = std::min<int64_t>(max_slabs, std::max<int64_t>(1, cdiv(4 * (int64_t)sms, gx)));
+    int64_t slabs = std::min<int64_t>(max_slabs, std::max<int64_t>(1, cdiv(4 * (int64_t)ctx.sm_count, gx)));
     slabs = std::min<int64_t>(slabs, 65535);
     int64_t slab_len = cdiv(cdiv(nb, slabs), kNnTile) * kNnTile;
     slabs = cdiv(nb, slab_len);
@@ -162,13 +151,13 @@ void mesh_sample(const float* verts, int64_t V, const int32_t* faces, int64_t F,
                  float* samples, int32_t* face_ids, cudaStream_t st) {
     P2S_CHECK(V > 0 && F > 0, "empty mesh");
     if (n <= 0) return;
-    auto& sc = scratch();
-    double* area = sc.area.as<double>((size_t)F);
-    double* cum = sc.cum.as<double>((size_t)F);
+    DeviceCtx& ctx = device_ctx();
+    double* area = ctx.mesh_area.as<double>((size_t)F);
+    double* cum = ctx.mesh_cum.as<double>((size_t)F);
     P2S_LAUNCH(face_area_kernel, (unsigned)cdiv(F, 256), 256, 0, st, verts, faces, F, V, area);
     size_t tmp_bytes = 0;
     P2S_CUDA(cub::DeviceScan::InclusiveSum(nullptr, tmp_bytes, area, cum, (int)F, st));
-    void* tmp = sc.cub_tmp.get(tmp_bytes);
+    void* tmp = ctx.mesh_cub.get(tmp_bytes);
     P2S_CUDA(cub::DeviceScan::InclusiveSum(tmp, tmp_bytes, area, cum, (int)F, st));
     g_launches.fetch_add(1, std::memory_order_relaxed);
     P2S_LAUNCH(mesh_sample_kernel, (unsigned)cdiv(n, 256), 256, 0, st, verts, faces, F, cum, n, seed, samples, face_ids);
@@ -183,9 +172,8 @@ void nn_distance(const float* a, int64_t na, const float* b, int64_t nb, float* 
 // out4 (host): sum a->b, sum b->a, max a->b, max b->a
 void chamfer_hausdorff(const float* a, int64_t na, const float* b, int64_t nb, double* out4_host, cudaStream_t st) {
     P2S_CHECK(na > 0 && nb > 0, "empty cloud");
-    auto& sc = scratch();
     // [0..1] f64 sums, then 2 x u32 maxima
-    double* red = sc.red.as<double>(3);
+    double* red = device_ctx().mesh_red.as<double>(3);
     P2S_CUDA(cudaMemsetAsync(red, 0, 3 * sizeof(double), st));
     unsigned int* mx = reinterpret_cast<unsigned int*>(red + 2);
     nn_core(a, na, b, nb, nullptr, nullptr, red + 0, mx + 0, st);

@@ -39,17 +39,10 @@ struct Model {
     cudaStream_t own_stream = nullptr;  // used by the *_host entry points
     DevBuf ws_net;                       // network activations
     DevBuf ws_io;                        // staged host inputs / assembled query batches
-    DevBuf ws_misc;
-    DevBuf ws_guard;
+    DevBuf ws_misc;                      // candidate list of the fused pipeline / gathered guard-band rows
+    DevBuf ws_guard;                     // guard-band index lists
     DevBuf ws_host;                      // device staging of host-call inputs/outputs
-    int64_t* guard_count_dev = nullptr;
     int64_t last_guard_count = 0;
-    // deferred guard band (fused pipeline): instead of recomputing inside every batch, forward_tc appends
-    // guard_base + i for every flagged query to guard_list; the caller recomputes them all at once
-    int32_t* guard_list = nullptr;
-    int* guard_list_count = nullptr;
-    int64_t guard_list_cap = 0;
-    int64_t guard_base = 0;
     float* debug_aux = nullptr;          // optional [B][kAuxStride]: R(9), feat_local_max(1024), feat_global_max(1024)
 };
 constexpr int kAuxStride = 2064;
@@ -63,13 +56,13 @@ void tc_build(Model& m);
 void tc_destroy(Model& m);
 void tc_profile_reset(Model& m, bool on);
 void tc_profile_get(Model& m, double* ms, int64_t* launches, double* flops);
-void forward_guard(Model& m, const float* patch, const float* sub, const float* query, int64_t B, float* logits, cudaStream_t st);
+// precise: split-precision operands (the guard-band recompute); fp16 operands otherwise
 void forward_tc(Model& m, const float* patch, const float* sub, const float* query, int64_t B,
-                float* logits, cudaStream_t st);
+                float* logits, cudaStream_t st, bool precise);
+void guard_flag(const float* logits, int64_t B, float band, int64_t base, int32_t* list, int* count, int64_t cap, cudaStream_t st);
 // fc_tc.cu
 bool fc_tc_supported(int N, int K);
 uint8_t* fc_tc_pack(const Layer& L, std::vector<void*>& allocs);
-void fc_tc_init();
 void launch_fc_tc(const float* A, int lda, const uint8_t* Wimg, const float* bias, float* C, int ldc,
                   int64_t M, int N, int K, bool relu, cudaStream_t st);
 uint8_t* fc_tc_pack_raw(const float* W, int N, int K, std::vector<void*>& allocs);
@@ -114,9 +107,6 @@ void op_add_row(float* x, const float* v, int64_t B, int C, cudaStream_t st);
 void op_sgd(float* p, const float* g, float* buf, int64_t n, float lr, float momentum, bool first, cudaStream_t st);
 void op_axpy(float* y, const float* x, float a, int64_t n, cudaStream_t st);
 void op_center(const float* in, const float* q, int64_t B, int npts, float* out, cudaStream_t st);
-// dispatch (api.cu)
-void forward(Model& m, const float* patch, const float* sub, const float* query, int64_t B,
-             float* logits, cudaStream_t st);
 
 // small shared kernels (net_fp32.cu), also used by the TC path for the per-query FC tails
 void launch_gemm_nt(const float* A, int64_t a_stride_z, int lda, const float* W, int64_t w_stride_z,

@@ -582,18 +582,6 @@ __global__ void guard_flag_kernel(const float* __restrict__ logits, int64_t B, f
         if (slot < cap) list[slot] = (int32_t)(base + i);
     }
 }
-__global__ void guard_gather_kernel(const float* __restrict__ src, const int32_t* __restrict__ list, int n, int row_floats, float* __restrict__ dst) {
-    int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= (int64_t)n * row_floats) return;
-    int i = (int)(e / row_floats), j = (int)(e % row_floats);
-    dst[e] = src[(int64_t)list[i] * row_floats + j];
-}
-__global__ void guard_scatter_kernel(const float* __restrict__ src, const int32_t* __restrict__ list, int n, float* __restrict__ logits) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    logits[(int64_t)list[i] * 2 + 0] = src[i * 2 + 0];
-    logits[(int64_t)list[i] * 2 + 1] = src[i * 2 + 1];
-}
 
 }  // namespace
 
@@ -628,7 +616,6 @@ struct TcWeights {
     const uint8_t* fold_img[2] = {nullptr, nullptr};
     const float* fold_bias[2] = {nullptr, nullptr};
     std::vector<void*> allocs;
-    int sm_count = 148;
     // profile of the dominant kernel (bench.py roofline)
     bool prof_on = false;
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> prof_events;
@@ -684,16 +671,17 @@ void launch_pass(Model& m, const TcStack& s, const Seg& s0, const Seg& s1, const
     p.out = out;
     p.wstats = nullptr;
     TcWeights& t = *m.tc;
+    DeviceCtx& ctx = device_ctx();
     static int wstats_on = -1;
     if (wstats_on < 0) { const char* e = getenv("P2S_TC_WAITSTATS"); wstats_on = (e && e[0] == '1') ? 1 : 0; }
-    static long long* wstats_dev = nullptr;
+    long long* wstats_dev = nullptr;
     if (wstats_on && !precise) {
-        if (!wstats_dev) P2S_CUDA(cudaMalloc(&wstats_dev, 6 * WS_SLOTS * sizeof(long long)));
+        wstats_dev = ctx.wait_stats.as<long long>(6 * WS_SLOTS);
         P2S_CUDA(cudaMemsetAsync(wstats_dev, 0, 6 * WS_SLOTS * sizeof(long long), st));
         p.wstats = wstats_dev;
     }
     const int split = precise ? Cfg<true>::kSplit : Cfg<false>::kSplit;
-    int streams = t.sm_count / split;
+    int streams = ctx.sm_count / split;
     if ((int64_t)streams > B) streams = (int)B;
     const int grid = streams * split;
     cudaEvent_t e0 = nullptr, e1 = nullptr;
@@ -704,8 +692,7 @@ void launch_pass(Model& m, const TcStack& s, const Seg& s0, const Seg& s1, const
     }
     if (precise) P2S_LAUNCH(pointnet_pass_kernel<true>, grid, kThreads, Cfg<true>::kSmemBytes, st, p);
     else if (wstats_on) {
-        static bool attr = false;
-        if (!attr) { P2S_CUDA(cudaFuncSetAttribute(pointnet_pass_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg<false>::kSmemBytes)); attr = true; }
+        ctx.set_max_dynamic_smem((const void*)pointnet_pass_kernel<false, true>, (int)Cfg<false>::kSmemBytes);
         P2S_LAUNCH((pointnet_pass_kernel<false, true>), grid, kThreads, Cfg<false>::kSmemBytes, st, p);
     } else P2S_LAUNCH(pointnet_pass_kernel<false>, grid, kThreads, Cfg<false>::kSmemBytes, st, p);
     if (wstats_on && !precise) {
@@ -713,8 +700,8 @@ void launch_pass(Model& m, const TcStack& s, const Seg& s0, const Seg& s1, const
         long long h[6 * WS_SLOTS];
         P2S_CUDA(cudaMemcpyAsync(h, wstats_dev, sizeof(h), cudaMemcpyDeviceToHost, st));
         P2S_CUDA(cudaStreamSynchronize(st));
-        static const char* roles[6] = {"big-issuer", "mid-issuer", "chain0", "chain1", "first-layer", "colmax"};
-        static const char* slots[WS_TOTAL] = {"act2_full", "d3_empty", "dmid_free", "dmid_ready", "act2_empty", "a_free", "d3_full"};
+        static const char* const roles[6] = {"big-issuer", "mid-issuer", "chain0", "chain1", "first-layer", "colmax"};
+        static const char* const slots[WS_TOTAL] = {"act2_full", "d3_empty", "dmid_free", "dmid_ready", "act2_empty", "a_free", "d3_full"};
         fprintf(stderr, "p2s waitstats: pass num_mid=%d perq=%d pts=%d+%d B=%lld precise=%d grid=%d\n", s.num_mid, perq_layer, s0.n, s1.n, (long long)B, (int)precise, grid);
         for (int r = 0; r < 6; ++r) {
             const double tot = (double)h[r * WS_SLOTS + WS_TOTAL];
@@ -743,11 +730,9 @@ void tc_build(Model& m) {
     P2S_CHECK(m.cfg.net_size == 1024, "tensor-core path needs net_size 1024");
     TcWeights* t = new TcWeights();
     m.tc = t;
-    cudaDeviceProp prop;
-    P2S_CUDA(cudaGetDeviceProperties(&prop, m.device));
-    t->sm_count = prop.multiProcessorCount;
-    P2S_CUDA(cudaFuncSetAttribute(pointnet_pass_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg<false>::kSmemBytes));
-    P2S_CUDA(cudaFuncSetAttribute(pointnet_pass_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg<true>::kSmemBytes));
+    DeviceCtx& ctx = device_ctx();
+    ctx.set_max_dynamic_smem((const void*)pointnet_pass_kernel<false>, (int)Cfg<false>::kSmemBytes);
+    ctx.set_max_dynamic_smem((const void*)pointnet_pass_kernel<true>, (int)Cfg<true>::kSmemBytes);
     auto build_stn = [&](TcStack& s, const Stn& stn, const Layer* c0a, const Layer* c0b) {
         // QSTN: x -> conv1(3->64) [layer 0] -> conv2 (64->128) -> conv3 ; STN64 on feat: conv0a [layer 0] -> conv0b -> conv1 -> conv2 -> conv3
         if (!c0a) {
@@ -781,7 +766,6 @@ void tc_build(Model& m) {
         s.w3_img = pack_w3(*t, f.conv3);
         s.b3 = f.conv3.b;
     };
-    fc_tc_init();
     // every FC layer but the QSTN's fc3 (256 -> 4) and fc4 (128 -> 2) runs on the tensor-core FC kernel; fc_tc_pack checks the shape
     auto mk_stn_fc = [&](const Stn& s) { TcStnFc r; r.fc1 = fc_tc_pack(s.fc1, t->allocs); r.fc2 = fc_tc_pack(s.fc2, t->allocs); return r; };
     if (m.shared_qstn) t->qstn_fc = mk_stn_fc(m.point_stn);
@@ -839,8 +823,8 @@ void tc_profile_get(Model& m, double* ms, int64_t* launches, double* flops) {
 
 // One pass of the network over B queries on tensor cores.  precise = split-precision operands everywhere
 // (the accurate path used for the guard band); fp16 operands otherwise.
-static void forward_tc_core(Model& m, const float* patch, const float* sub, const float* query, int64_t B,
-                            float* logits, cudaStream_t st, bool precise) {
+void forward_tc(Model& m, const float* patch, const float* sub, const float* query, int64_t B,
+                float* logits, cudaStream_t st, bool precise) {
     TcWeights& t = *m.tc;
     const int P = m.cfg.points_per_patch, S = m.cfg.sub_sample_size;
     const int64_t Bc_max = 8192;
@@ -916,41 +900,9 @@ static void forward_tc_core(Model& m, const float* patch, const float* sub, cons
     }
 }
 
-// accurate recompute used for the guard band: the split-precision tensor-core path
-void forward_guard(Model& m, const float* patch, const float* sub, const float* query, int64_t B, float* logits, cudaStream_t st) {
-    forward_tc_core(m, patch, sub, query, B, logits, st, true);
-}
-
-void forward_tc(Model& m, const float* patch, const float* sub, const float* query, int64_t B,
-                float* logits, cudaStream_t st) {
-    const int P = m.cfg.points_per_patch, S = m.cfg.sub_sample_size;
-    forward_tc_core(m, patch, sub, query, B, logits, st, false);
-
-    // guard band: queries whose sign logit is too close to 0 for fp16-operand arithmetic are recomputed in fp32
-    if (m.guard_band > 0.f && m.guard_list) {
-        // deferred: only record which queries fall into the band (the fused pipeline recomputes them in one batch)
-        P2S_LAUNCH(guard_flag_kernel, (unsigned)cdiv(B, 256), 256, 0, st, logits, B, m.guard_band, m.guard_list, m.guard_list_count, m.guard_base, m.guard_list_cap);
-    } else if (m.guard_band > 0.f) {
-        StageScope ts_guard("net: guard-band fp32 recompute", st);
-        int32_t* list = m.ws_guard.as<int32_t>((size_t)B + 64);
-        int* count = reinterpret_cast<int*>(list + B);
-        P2S_CUDA(cudaMemsetAsync(count, 0, sizeof(int), st));
-        P2S_LAUNCH(guard_flag_kernel, (unsigned)cdiv(B, 256), 256, 0, st, logits, B, m.guard_band, list, count, (int64_t)0, B);
-        int n = 0;
-        P2S_CUDA(cudaMemcpyAsync(&n, count, sizeof(int), cudaMemcpyDeviceToHost, st));
-        P2S_CUDA(cudaStreamSynchronize(st));
-        m.last_guard_count += n;
-        if (n > 0) {
-            const size_t rowp = (size_t)P * 3, rows = (size_t)S * 3;
-            float* gbuf = m.ws_misc.as<float>((size_t)n * (rowp + rows + 3 + 2) + 64);
-            float* gp = gbuf; float* gs = gp + (size_t)n * rowp; float* gq = gs + (size_t)n * rows; float* gl = gq + ((size_t)n * 3 + 3) / 4 * 4;
-            P2S_LAUNCH(guard_gather_kernel, (unsigned)cdiv((int64_t)n * rowp, 256), 256, 0, st, patch, list, n, (int)rowp, gp);
-            P2S_LAUNCH(guard_gather_kernel, (unsigned)cdiv((int64_t)n * rows, 256), 256, 0, st, sub, list, n, (int)rows, gs);
-            P2S_LAUNCH(guard_gather_kernel, (unsigned)cdiv((int64_t)n * 3, 256), 256, 0, st, query, list, n, 3, gq);
-            forward_guard(m, gp, gs, gq, n, gl, st);
-            P2S_LAUNCH(guard_scatter_kernel, (unsigned)cdiv(n, 256), 256, 0, st, gl, list, n, logits);
-        }
-    }
+// appends base + i to list[0..cap) for every query i < B whose |sign logit| < band; *count counts them
+void guard_flag(const float* logits, int64_t B, float band, int64_t base, int32_t* list, int* count, int64_t cap, cudaStream_t st) {
+    P2S_LAUNCH(guard_flag_kernel, (unsigned)cdiv(B, 256), 256, 0, st, logits, B, band, list, count, base, cap);
 }
 
 }  // namespace p2s

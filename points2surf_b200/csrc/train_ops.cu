@@ -401,17 +401,6 @@ __global__ void center_kernel(const float* __restrict__ in, const float* __restr
     out[e] = in[e] - q[b * 3 + e % 3];
 }
 
-int sm_count() {
-    static int n = 0;
-    if (!n) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-        if (n <= 0) n = 148;
-    }
-    return n;
-}
-
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------- host launchers
@@ -427,7 +416,7 @@ void op_gemm_tn(const float* A, int64_t a_stride_z, int lda, const float* B, int
     const int tiles = (int)(cdiv(N, kTnN) * cdiv(K, kTnK)) * batch;
     int splits = 1;
     if (M > 2048) {
-        splits = (int)std::min<int64_t>(cdiv(M, 1024), std::max<int64_t>(1, cdiv(4 * (int64_t)sm_count(), tiles)));
+        splits = (int)std::min<int64_t>(cdiv(M, 1024), std::max<int64_t>(1, cdiv(4 * (int64_t)device_ctx().sm_count, tiles)));
     }
     int rows = (int)(cdiv(cdiv(M, splits), kTnM) * kTnM);
     splits = (int)cdiv(M, rows);
@@ -455,7 +444,7 @@ void op_transpose(const float* in, float* out, int rows, int cols, int batch, cu
 
 static void col_reduce_grid(int64_t M, int C, dim3& g, int64_t& rows_per_block) {
     int64_t cx = cdiv(C, 32);
-    int64_t want = std::max<int64_t>(1, cdiv(8 * (int64_t)sm_count(), cx));
+    int64_t want = std::max<int64_t>(1, cdiv(8 * (int64_t)device_ctx().sm_count, cx));
     rows_per_block = std::max<int64_t>(64, cdiv(M, want));
     rows_per_block = std::min<int64_t>(rows_per_block, 4096);
     rows_per_block = std::max<int64_t>(rows_per_block, cdiv(M, 65535));
@@ -467,7 +456,7 @@ static void rowwise_grid(int64_t M, int C, dim3& blk, dim3& g, int64_t& rows_per
     const int tx = C >= 128 ? 128 : (C >= 64 ? 64 : 32);
     blk = dim3(tx, 256 / tx);
     const int64_t cx = cdiv(C, tx);
-    const int64_t want = std::max<int64_t>(1, cdiv(16 * (int64_t)sm_count(), cx));
+    const int64_t want = std::max<int64_t>(1, cdiv(16 * (int64_t)device_ctx().sm_count, cx));
     rows_per_block = std::max<int64_t>(4 * blk.y, cdiv(M, want));
     rows_per_block = std::max<int64_t>(rows_per_block, cdiv(M, 65535));
     g = dim3((unsigned)cx, (unsigned)cdiv(M, rows_per_block));

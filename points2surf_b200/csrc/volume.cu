@@ -579,8 +579,6 @@ __global__ void finalize_kernel(float* __restrict__ vol, const uint8_t* __restri
     vol[v] = x;
 }
 
-thread_local DevBuf t_vol_ws;
-
 }  // namespace
 
 void sdf_from_logits(const float* logits, const float* radius, int64_t B, float* sdf, cudaStream_t st) {
@@ -608,7 +606,8 @@ void sdf_to_volume(const int32_t* lin_idx, const float* sdf, int64_t Q, int res,
     const size_t off_lists = off; off += 3 * nt4 * sizeof(int);
     const size_t off_vz = off; off += nt4 * sizeof(int);
     const size_t off_flags = off; off += 2 * nt4;
-    uint8_t* base = (uint8_t*)t_vol_ws.get(off);
+    DeviceCtx& ctx = device_ctx();
+    uint8_t* base = (uint8_t*)ctx.vol_ws.get(off);
     Ctrl* ctrl = (Ctrl*)base;
     pp.ctrl = ctrl;
     pp.buf[0] = base + off_A; pp.buf[1] = base + off_B;
@@ -637,16 +636,14 @@ void sdf_to_volume(const int32_t* lin_idx, const float* sdf, int64_t Q, int res,
     const size_t smem_generic = (size_t)((X0 * Y0 * ZS + 15) & ~15) + (size_t)((X0 * Y0 * TZ + 15) & ~15) + (size_t)X0 * TY * TZ * 2;
     const size_t smem_fast = 4 * ((size_t)X0 * Y0 * (ZS / 4) + (size_t)TX * TY * 8 + (size_t)X0 * Y0 * 8 + (size_t)X0 * TY * 8);
     const size_t smem = pp.fast ? smem_fast : smem_generic;
-    int dev_id = 0, sms = 148, per_sm = 0;
-    P2S_CUDA(cudaGetDevice(&dev_id));
-    P2S_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev_id));
+    int per_sm = 0;
     const bool s5 = pp.fast && sigma == 5;
     const void* kfn = s5 ? (const void*)propagate_kernel<true> : (const void*)propagate_kernel<false>;
-    P2S_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ctx.set_max_dynamic_smem(kfn, (int)smem);
     if (s5) P2S_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, propagate_kernel<true>, kPropThreads, smem));
     else P2S_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, propagate_kernel<false>, kPropThreads, smem));
     P2S_CHECK(per_sm >= 1, "sign propagation kernel does not fit on an SM");
-    const unsigned grid = (unsigned)std::max(1, std::min(numTiles, sms * per_sm));
+    const unsigned grid = (unsigned)std::max(1, std::min(numTiles, ctx.sm_count * per_sm));
     void* args[] = {&pp};
     P2S_CUDA(cudaLaunchCooperativeKernel(kfn, dim3(grid), dim3(kPropThreads), args, smem, st));
     g_launches.fetch_add(1, std::memory_order_relaxed);

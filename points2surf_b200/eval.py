@@ -50,7 +50,7 @@ def parse_arguments(args=None):
     parser.add_argument('--workers', type=int, default=0, help='unused: there is no DataLoader on this path')
     parser.add_argument('--cache_capacity', type=int, default=100, help='unused (kept for CLI compatibility)')
     parser.add_argument('--precision', type=str, default='tc', choices=['tc', 'fp32'], help='tensor-core fp16/fp32-acc or fp32 FMA')
-    parser.add_argument('--guard_band', type=float, default=0.05, help='|sign logit| below which a query is recomputed in fp32')
+    parser.add_argument('--guard_band', type=float, default=0.05, help='|sign logit| below which a query is recomputed in split precision')
     opt = parser.parse_args(args=args)
     if len(opt.dataset) == 1:
         opt.dataset = opt.dataset[0]

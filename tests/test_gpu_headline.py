@@ -110,6 +110,26 @@ def test_headline_vanilla_res128_all_queries():
     eng.close()
 
 
+def test_guard_band_recomputes_every_query_over_several_batches():
+    """A guard band wider than any |sign logit|: every batch flags all its queries into the slab-wide list (at the batch's
+    offset), and all of them are recomputed in split precision, in batches of the same size.  The result must not depend on
+    the batch size."""
+    cloud = synth.make_cloud('sphere', 10000, seed=0)
+    sd, eng = bench_engine('vanilla')
+    eng.set_precision('tc', guard_band=1e9)
+    lin, sdf = eng.reconstruct(cu(cloud), 128, 3, 0, SEED)
+    Q = lin.numel()
+    assert eng.last_guard_count() == Q
+    lin2, sdf2 = eng.reconstruct(cu(cloud), 128, 3, 0, SEED, batch=3000)
+    assert Q > 4 * 3000
+    assert eng.last_guard_count() == Q
+    assert torch.equal(lin, lin2)
+    a, b = sdf.cpu().numpy(), sdf2.cpu().numpy()
+    assert np.array_equal(np.sign(a), np.sign(b))
+    assert np.abs(a - b).max() <= 1e-6
+    eng.close()
+
+
 def test_headline_vanilla_res256_slab():
     """The bench line's own resolution: a 20 000-query slab (three default batches) of the res-256 band."""
     cloud = synth.make_cloud('sphere', 10000, seed=0)
